@@ -7,6 +7,7 @@
     python bench.py --impl reference ...      # the reference's CPU implementation on the host cores
     python bench.py --workload kuka|cspr ...  # BASELINE configs[2] / configs[3] (defaults: 4096 / 65536 paths)
     python bench.py --total 1048576 ...       # strong scaling: the 2^20-path batch split over the ranks
+    python bench.py --dump-outputs DIR ...    # also write the last timed step's results as DIR/*.npy (rank 0)
 
 Workloads (seeded synthetic paths, batotp_b200/synth.py; recipes of the reference's own Octave generators):
   gen7dof (default)  configs[4]: GEN7DOF, 20 knots U[0,5]^7 -> 400 pts, joint velocity / acceleration limits;
@@ -92,7 +93,16 @@ def parse():
     ap.add_argument("--pitched", action="store_true",
                     help="e2e leg: rows at the pitch of the longest trajectory instead of the ragged layout")
     ap.add_argument("--lib", default=None, help="experiments only: alternative build of libbatotp_cuda.so")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0, at most "
+                         "64 MB): the resident leg's per-trajectory values and the host-buffer leg's output rows of a "
+                         "fixed sample of trajectories, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs: only the b200 arm returns outputs")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -325,6 +335,52 @@ def latency_block(ctx):
     return out
 
 
+# ----------------------------------------------------------------------------- output dump
+DUMP_BYTES = 64_000_000
+SCALARS = ("status", "n_rev", "n_fwd", "n_out", "n_cart_out", "n_grid", "t_total", "t_rev", "s_last_sec", "out_sres")
+
+
+def dump_outputs(d, res_s, res_e, e2e_first):
+    """--dump-outputs: the arrays the timed legs returned in their last step, as .npy files in d.
+    Per-trajectory values of the resident leg (float64, exact for the integer ones) for every trajectory of the batch,
+    or for a seeded sample when the batch is too large; traj_index.npy holds the trajectory indices.  Output rows of
+    the host-buffer leg (float32, as returned): the trajectories res_e holds (those from e2e_first on), taken in a
+    seeded order for as long as the total stays within DUMP_BYTES; each of theta_out / trq_out / cart_out is the
+    concatenation of the sampled trajectories' [rows, n] blocks; rows_index.npy holds their trajectory indices,
+    rows_n.npy their n (cart_n.npy that of the Cartesian blocks)."""
+    os.makedirs(d, exist_ok=True)
+    B = res_s.B
+    per_traj = 8 * (len(SCALARS) + 1)
+    idx = np.arange(B)
+    if B * per_traj > DUMP_BYTES // 2:
+        idx = np.sort(np.random.default_rng(1).permutation(B)[:DUMP_BYTES // 2 // per_traj])
+    np.save(os.path.join(d, "traj_index.npy"), idx.astype(np.float64))
+    for nm in SCALARS:
+        np.save(os.path.join(d, nm + ".npy"), getattr(res_s, nm)[idx].astype(np.float64))
+    if res_e is None:
+        return
+    left = DUMP_BYTES - per_traj * len(idx) - (1 << 16)  # (1 << 16: the .npy headers)
+    names = [nm for nm in ("theta_out", "trq_out", "cart_out") if getattr(res_e, nm) is not None]
+    rows = {nm: [] for nm in names + ["rows_index", "rows_n"] + (["cart_n"] if "cart_out" in names else [])}
+    for b in np.random.default_rng(2).permutation(B - e2e_first):
+        blk = {nm: res_e.rows(b, nm) for nm in names if nm != "cart_out"}
+        if "cart_out" in names:
+            blk["cart_out"] = res_e.cart_out[b, :res_e.Cin, :int(res_e.n_cart_out[b])]
+        cost = sum(a.nbytes for a in blk.values()) + 24
+        if cost > left:
+            break
+        left -= cost
+        for nm, a in blk.items():
+            rows[nm].append(a.ravel())
+        rows["rows_index"].append([e2e_first + b])
+        rows["rows_n"].append([blk["theta_out"].shape[1]])
+        if "cart_out" in blk:
+            rows["cart_n"].append([blk["cart_out"].shape[1]])
+    for nm, parts in rows.items():
+        a = np.concatenate(parts) if parts else np.zeros(0, np.float32)
+        np.save(os.path.join(d, nm + ".npy"), a if nm in names else a.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- B200 arm
 def main_b200(args):
     import torch
@@ -393,12 +449,14 @@ def main_b200(args):
     barrier()
     ctx.stats_reset()
     clk = ClockSampler(local)
-    ctx.timer_start()
-    for _ in range(args.steps):
-        step_resident()
-    ms = ctx.timer_stop_ms()
-    barrier()
-    clocks = clk.stop()
+    try:  # the sampler is a child process: it must not outlive a failed step
+        ctx.timer_start()
+        for _ in range(args.steps):
+            step_resident()
+        ms = ctx.timer_stop_ms()
+        barrier()
+    finally:
+        clocks = clk.stop()
     st = ctx.stats()
     slog = ctx.sweep_log()
     ms = max_over_ranks(ms)
@@ -515,6 +573,9 @@ def main_b200(args):
                         "float32 rows (%s) + per-trajectory scalars copied back; bytes per rank"
                         % (nsl, sl, "ragged: every trajectory at its own length, the payload of trajWriteBIN" if ragged
                            else "pitch %d points = the longest trajectory" % out_cap))
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res_s, None if e2e is None else res_e, (B - 1) // sl * sl)
 
     line = None
     if rank == 0:

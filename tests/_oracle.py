@@ -2,12 +2,15 @@
 
 * ``Oracle``  — oracle/_build/libba_oracle.so, the C restatement (always buildable).
 * ``Ref``     — oracle/_ref/libbatotp_ref.so, the unmodified reference sources compiled
-                in place with the Eigen stand-in (present when /root/reference was
-                available at build time, or when the prebuilt file travelled to the box).
+                in place with the Eigen stand-in (``make -C oracle ref REF=<reference tree>``).
+* ``RefSide`` — the reference's side of a comparison: ``Ref`` where it is built, the digests
+                of its results stored in tests/golden/reference_digests.json elsewhere.
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -20,6 +23,7 @@ from batotp_b200.config import BatotpCfg  # noqa: E402
 
 ORC_SO = os.path.join(ROOT, "oracle", "_build", "libba_oracle.so")
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libbatotp_ref.so")
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_digests.json")
 
 _dp = C.POINTER(C.c_double)
 _fp = C.POINTER(C.c_float)
@@ -79,6 +83,59 @@ _ref = None
 
 def ref_available() -> bool:
     return os.path.exists(REF_SO)
+
+
+def digest(value) -> str:
+    """dtype, shape and sha256[:16] of a result's bytes (Python numbers as float64, bytes as uint8)."""
+    if isinstance(value, bytes):
+        a = np.frombuffer(value, np.uint8)
+    elif isinstance(value, np.ndarray):
+        a = np.ascontiguousarray(value)
+    else:
+        a = np.asarray(value, dtype=np.float64)
+    return "%s%s:%s" % (a.dtype.str, list(a.shape), hashlib.sha256(a.tobytes()).hexdigest()[:16])
+
+
+class RefSide:
+    """The reference's side of one test case's comparisons.
+
+    Where oracle/_ref is built the reference library itself runs: ``same`` compares its result with the value and
+    checks it against the stored digest (with BATOTP_RECORD_REF_DIGESTS=1 it stores the digest instead; ``save``
+    writes the file).  Elsewhere the reference is not called at all and ``same`` compares the value's digest with
+    the stored one, so the comparisons hold on every checkout."""
+
+    def __init__(self, case: str):
+        self.case = case
+        self.live = ref_available()
+        self.record = self.live and os.environ.get("BATOTP_RECORD_REF_DIGESTS") == "1"
+        self.stored = json.load(open(REF_DIGESTS)).get(case, {}) if os.path.exists(REF_DIGESTS) else {}
+        self.seen = {}
+
+    def call(self, fn):
+        """fn() on the live reference; None where the reference is not built."""
+        return fn() if self.live else None
+
+    def same(self, key: str, ref_fn, value) -> bool:
+        """Is the reference's result (ref_fn(), called only on the live reference) bit for bit ``value``?"""
+        if not self.live:
+            assert key in self.stored, "no stored reference result %s / %s" % (self.case, key)
+            return self.stored[key] == digest(value)
+        x = ref_fn()
+        if self.record:
+            self.seen[key] = digest(x)
+        else:
+            assert self.stored.get(key, digest(x)) == digest(x), \
+                "%s: %s differs from the stored reference digest" % (self.case, key)
+        return x == value if isinstance(x, bytes) else bool(np.array_equal(x, value))
+
+    def save(self):
+        if not self.record:
+            return
+        db = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+        db[self.case] = self.seen
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(db, f, indent=0, sort_keys=True)
+            f.write("\n")
 
 
 def ref_lib():

@@ -68,7 +68,6 @@ def load(path: Optional[str] = None):
     L.batotp_cuda_set_tail_overlap.argtypes = [C.c_void_p, C.c_int]
     L.batotp_cuda_set_step_hint.argtypes = [C.c_void_p, C.c_int]
     L.batotp_cuda_set_dyn_callback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-    L.batotp_cuda_set_pipeline.argtypes = [C.c_void_p, C.c_int]
     L.batotp_cuda_set_sweep_kernel.argtypes = [C.c_void_p, C.c_int]
     L.batotp_cuda_set_walker_kernel.argtypes = [C.c_void_p, C.c_int]
     L.batotp_cuda_launch_count.argtypes = [C.c_void_p]
@@ -255,8 +254,9 @@ class Context:
         self.L.batotp_cuda_set_walker_kernel(self.h, mode)
 
     def set_pipeline(self, on: int):
-        """0 off, 1 automatic, n > 1: two-context pipeline with chunks of n trajectories."""
-        self.L.batotp_cuda_set_pipeline(self.h, int(on))
+        """Kept because bench.py passes --pipeline: 0 does nothing, anything else raises."""
+        if int(on) != 0:
+            raise NativeError("the two-context chunk pipeline was removed from the library (see DESIGN.md)")
 
     def set_dyn_callback(self, fn, user=None):
         """fn: address of (or ctypes pointer to) a batotp_dyn_fn; None switches it off."""

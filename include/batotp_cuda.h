@@ -69,15 +69,6 @@ int batotp_cuda_set_step_hint(batotp_handle h, int n);
  * workspaces, one host thread), beside the output / input phases of the full chunks instead of after them.
  * Results are identical either way; 0 switches it off (one context, chunks strictly one after the other) */
 int batotp_cuda_set_tail_overlap(batotp_handle h, int on);
-/* two-context pipeline of batotp_cuda_optimize_batch (default OFF - on a B200 it measured slower than the tail
- * overlap, see DESIGN.md: the sweeps of the two contexts cannot share an SM's register file and a sweep's duration
- * hardly depends on the chunk size; kept as a tuning option.  1 = automatic chunking, batches of more than one
- * sweep wave only): chunks of two sweep CTAs per SM alternate between the context and a second one inside the
- * library (own streams, workspaces and host thread), so that the latency-bound sweep of one chunk runs beside the
- * bandwidth-bound input / output phases of its neighbours.  Results are identical either way; 0 = one context,
- * chunks of three sweep CTAs per SM strictly one after the other (with the tail overlap above); n > 1 = pipeline
- * with chunks of n trajectories whatever the batch size (tuning). */
-int batotp_cuda_set_pipeline(batotp_handle h, int on);
 /* number of kernels launched by this context since creation (for the benchmark's gpu_launches) */
 long batotp_cuda_launch_count(batotp_handle h);
 /* measurement hooks for bench.py.

@@ -204,7 +204,7 @@ struct batotp_ctx {
   DevCfg cfg;
   bool haveCfg = false;
   Ws w;
-  int capB = 0, capNc = 0, capSc = 0, capR = 0, capRT = 0;
+  int capB = 0, capNc = 0, capSc = 0, capR = 0, capC = 0, capRT = 0;
   bool capTrq = false;
   std::vector<void *> wsAllocs;   // chunk-resident arrays
   size_t wsBytes = 0, outBytes = 0;  // bytes held by wsAllocs / outAllocs
@@ -271,8 +271,8 @@ struct batotp_ctx {
   int setNext = 0;           // the staging sets rotate across sub-chunks AND chunks
   cudaStream_t copyStream = 0;
   double *d_cartOutD = nullptr;
-  double *d_outD = nullptr;  // [Bo][R+J][OutC] FP64 final rows (keepF64)
-  double *o_mS = nullptr, *o_sOut = nullptr, *o_tauO = nullptr, *o_O5 = nullptr, *o_OA = nullptr, *o_OM = nullptr;
+  double *d_outD = nullptr;  // [Bo][J+C+J][OutC] FP64 final rows (keepF64)
+  double *o_sOut = nullptr, *o_tauO = nullptr, *o_O5 = nullptr, *o_OA = nullptr, *o_OM = nullptr;
   double *o_OD = nullptr, *o_OD2 = nullptr, *o_Trq = nullptr, *o_Trq2 = nullptr, *o_TrqM = nullptr;
   int *o_segO = nullptr;
   bool keepF64 = false, capKeep = false, capFused = false;
@@ -526,7 +526,7 @@ int final_cap(const batotp_ctx *h, int Sc, int Os) {
 // bytes of chunk-resident workspace per trajectory (the arrays of ensure_ws)
 size_t chunk_bytes_per_traj(const DevCfg &c, int Nc, int Sc) {
   const size_t n = (size_t)Nc, sc = (size_t)Sc;
-  size_t per = 3 * (size_t)c.R * n * 8 + n * 8 + 2 * n * 8 + n * (size_t)c.RT * 32 + 4 * sc * 8 + 2 * sc + sizeof(TrajState);
+  size_t per = 3 * (size_t)c.R * n * 8 + n * 8 + 2 * n * 8 + n * (size_t)c.RT * 32 + 5 * sc * 8 + 2 * sc + sizeof(TrajState);
   if (c.trqOn) per += 2 * (size_t)4 * c.J * n * 8 + 2 * (size_t)c.R * n * 8;
   return per;
 }
@@ -539,12 +539,12 @@ size_t out_bytes_per_traj(const batotp_ctx *h, int Sc) {
   size_t Os = Oc;
   if (!trq && smooth_uniform_on(h)) Os = (size_t)(Oc / c.c.out_smooth_fact) + 16;
   const size_t OutC = (size_t)final_cap(h, Sc, (int)Os), R = (size_t)c.R;
-  size_t per = (size_t)Sc * 8 + Oc * 20 + (fused_out(h) ? 0 : R * Oc * 8) + 2 * R * Os * 8;
+  size_t per = Oc * 20 + (fused_out(h) ? 0 : R * Oc * 8) + 2 * R * Os * 8;
   if (trq) per += 2 * R * Oc * 8 + 3 * (size_t)MAXD * Oc * 8;
   per += 2 * ((size_t)c.J * OutC * 4 + (size_t)std::max(c.Cin, 1) * OutC * 4 + (trq ? (size_t)c.J * OutC * 4 : 0) +
               4 * (size_t)Sc * 4);
   if (c.C == 7) per += 7 * OutC * 8;
-  if (h->keepF64) per += (R + c.J) * OutC * 8;
+  if (h->keepF64) per += (size_t)(c.J + c.C + c.J) * OutC * 8;
   return per;
 }
 
@@ -554,8 +554,8 @@ void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
   const bool trq = c.trqOn != 0;
   // (with a step hint the capacity asked for is taken literally, not "at least")
   const bool scOk = h->stepHint > 0 ? (Sc == h->capSc) : (Sc <= h->capSc);
-  if (B <= h->capB && Nc <= h->capNc && scOk && c.R == h->capR && c.RT == h->capRT && trq == h->capTrq &&
-      c.J == h->w.AD) {
+  if (B <= h->capB && Nc <= h->capNc && scOk && c.R == h->capR && c.C == h->capC && c.RT == h->capRT &&
+      trq == h->capTrq && c.J == h->w.AD) {
     h->w.B = B;
     return;
   }
@@ -607,6 +607,7 @@ void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
   w.hist = ws_alloc<double>(h, b * 4 * Sc);
   w.flags = ws_alloc<unsigned char>(h, b * 2 * Sc);
   w.st = ws_alloc<TrajState>(h, b);
+  w.mS = ws_alloc<double>(h, b * Sc);
   if (trq) {
     w.A = ws_alloc<double>(h, b * 4 * w.AD * Nc);
     w.AM = ws_alloc<double>(h, b * 4 * w.AD * Nc);
@@ -620,6 +621,7 @@ void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
   h->capNc = Nc;
   h->capSc = Sc;
   h->capR = R;
+  h->capC = c.C;
   h->capRT = RT;
   h->capTrq = trq;
   ensure_tabs(h, std::max(Nc, Sc) + 8);
@@ -654,7 +656,6 @@ void ensure_out(batotp_ctx *h, int Bo, int minOutC = 0) {
     h->allocPhase = 1;
     const size_t b = (size_t)Bo;
     const int R = c.R;
-    h->o_mS = out_alloc<double>(h, b * Sc);
     h->o_sOut = out_alloc<double>(h, b * Oc);
     h->o_segO = out_alloc<int>(h, b * Oc);
     h->o_tauO = out_alloc<double>(h, b * Oc);
@@ -680,7 +681,7 @@ void ensure_out(batotp_ctx *h, int Bo, int minOutC = 0) {
     h->capHistPitch = histP;
     select_out_set(h, 0);
     h->d_cartOutD = (c.C == 7) ? out_alloc<double>(h, b * 7 * OutC) : nullptr;
-    h->d_outD = h->keepF64 ? out_alloc<double>(h, b * (R + c.J) * OutC) : nullptr;
+    h->d_outD = h->keepF64 ? out_alloc<double>(h, b * (c.J + c.C + c.J) * OutC) : nullptr;  // k_out_pack's layout
     h->capBo = Bo;
     h->capOc = Oc;
     h->capOs = Os;
@@ -693,7 +694,6 @@ void ensure_out(batotp_ctx *h, int Bo, int minOutC = 0) {
   w.Oc = h->capOc;
   w.Os = h->capOs;
   w.OutC = h->capOutC;
-  w.mS = h->o_mS;
   w.sOut = h->o_sOut;
   w.segO = h->o_segO;
   w.tauO = h->o_tauO;
@@ -718,7 +718,12 @@ void set_cfg(batotp_ctx *h, const batotp_cfg *cfg) {
   d.cartOn = (cfg->is_cart_vel_on || cfg->is_cart_acc_on) ? 1 : 0;
   d.trqOn = cfg->is_trq_on ? 1 : 0;
   if (d.C < 3) d.C = 3;  // adjust_s / interpSpecial always read cart rows 0..2 (ba.cpp:463, 697)
-  d.R = d.J + d.C;
+  // A joint-only generic robot (no kinematic model, joint path, no Cartesian or torque limits) has Cartesian rows
+  // that are zero throughout (ba.cpp:245-280 with no fwdKin): only its joint rows are stored, and the kernels read
+  // the Cartesian rows as a literal 0.0.  (isInterpOnly re-samples and returns whatever rows the input had.)
+  const bool jointOnly = cfg->robot_type == BATOTP_GENJNT && cfg->path_type == BATOTP_JOINT && !d.cartOn && !d.trqOn &&
+                         !cfg->is_interp_only;
+  d.R = jointOnly ? d.J : d.J + d.C;
   d.RT = d.J + (d.cartOn ? 3 : 0) + (d.trqOn ? 4 * d.J : 0);
   d.quadThresh = cfg->cart_thresh * cfg->cart_thresh;
   d.pm = h->pm;
@@ -881,6 +886,7 @@ void apply_kinematics(batotp_ctx *h, int where) {
   const int b0 = over ? h->w.b0 : 0;
   const int mode = kin_mode(h, where);
   if (mode == 0) return;
+  if (mode == 3 && c.R == c.J) return;  // the zeroed Cartesian rows are not stored
   if (mode == 1 && c.c.trig_mode == 2) {
     host_rows_apply(h, base, npts, nb, b0, over, 1);
     return;
@@ -1160,13 +1166,15 @@ int do_interp_input(batotp_ctx *h, bool haveN0, bool planSync) {
       BATOTP_LAUNCH_WARP(k_march_group, dim3((unsigned)(((long long)B * MG + 127) / 128)), dim3(128), 0, h->stream, w);
       g_check_launch();
       h->launches++;
-    } else if (c.J == 7 && c.C == 3)
+    } else if (c.J == 7 && c.R == 7)
+      LAUNCH_T(h, (k_march<7, 0>), B, w);
+    else if (c.J == 7 && c.R == 10)
       LAUNCH_T(h, (k_march<7, 3>), B, w);
-    else if (c.J == 6 && c.C == 7)
+    else if (c.J == 6 && c.R == 13)
       LAUNCH_T(h, (k_march<6, 7>), B, w);
-    else if (c.J == 3 && c.C == 3)
+    else if (c.J == 3 && c.R == 6)
       LAUNCH_T(h, (k_march<3, 3>), B, w);
-    else if (c.J == 2 && c.C == 3)
+    else if (c.J == 2 && c.R == 5)
       LAUNCH_T(h, (k_march<2, 3>), B, w);
     else
       LAUNCH_T(h, (k_march<0, 0>), B, w);
@@ -1285,7 +1293,9 @@ void do_interp_output(batotp_ctx *h, int b0, int Bo) {
   // launch extents from the longest trajectory of the chunk rather than from the capacities
   const int lOc = std::min(w.Oc, oversample_cap(h, std::max(h->mxSteps, 4)));
   const int lOs = (w.Os == w.Oc) ? lOc : std::min(w.Os, (int)(lOc / c.c.out_smooth_fact) + 16);
-  LAUNCH_T(h, k_out_plan, Bo, w, t);
+  // s(t) of the whole resident chunk is planned with its first sub-chunk: one launch of the sequential solve over
+  // the chunk's trajectories instead of one per sub-chunk (mS is chunk-resident, [B][Sc])
+  if (b0 == 0) LAUNCH_T(h, k_out_plan, h->B, w, t);
   {  // s(t) at the oversampled sites and their segments, 32x32 tiles
     const long long rows = cdiv(lOc, 32);
     const long long gy = std::min<long long>(rows, 32768), gz = (rows + gy - 1) / gy;
@@ -2734,6 +2744,11 @@ int batotp_cuda_get_f64(batotp_handle h, const char *name, int traj, int row, do
       if (buf && cap > 0) buf[0] = v;
       return 1;
     }
+    if ((n == "cartC_y" || n == "cartC_m") && c.R == c.J) {  // Cartesian rows that are not stored: zeros
+      if (s.status & ST_FATAL_MASK) return 0;
+      for (int i = 0; buf && i < std::min(s.nPtsC, cap); ++i) buf[i] = 0.0;
+      return s.nPtsC;
+    }
     if (n == "thetaC_y") { src = prow(w.P, row); stride = pst; len = s.nPtsC; }
     else if (n == "thetaC_m") { src = prow(w.M, row); stride = pst; len = s.nPtsC; }
     else if (n == "cartC_y") { src = prow(w.P, c.J + row); stride = pst; len = s.nPtsC; }
@@ -2748,10 +2763,10 @@ int batotp_cuda_get_f64(batotp_handle h, const char *name, int traj, int row, do
     else if (h->phase >= 3 && n == "sdot_fwd") { src = w.hist + (size_t)traj * 4 * w.Sc + 3 * (size_t)w.Sc; len = s.nFwd; }
     else if (h->phase >= 4 && h->d_outD && traj >= w.b0 && traj < w.b0 + w.Bo &&
              (n == "theta_out" || n == "cart_out" || n == "trq_out")) {
-      const int rows = c.R + c.J, bl = traj - w.b0;
+      const int rows = c.J + c.C + c.J, bl = traj - w.b0;  // k_out_pack's layout of outD
       auto orow_ = [&](int r) { return h->d_outD + ((size_t)bl * rows + r) * w.OutC; };
       if (n == "theta_out") { src = orow_(row); len = s.nOut; }
-      else if (n == "trq_out") { src = orow_(c.R + row); len = s.nOut; }
+      else if (n == "trq_out") { src = orow_(c.J + c.C + row); len = s.nOut; }
       else {
         len = s.nCartOut;
         if (c.C == 7 && row >= 3) {  // q2aaVect (ba.cpp:382-403) with the host libm

@@ -214,7 +214,7 @@ __global__ void k_in_load(WSP, const T *theta, const T *cart, const int *n0, con
   if (i >= n) return;
   double *dst = w.P + ((size_t)i * w.B + b) * w.R;
   for (int j = 0; j < CFG.J; ++j) dst[j] = theta ? (double)theta[((size_t)b * CFG.J + j) * n0max + i] : 0.0;
-  for (int j = 0; j < CFG.C; ++j) {
+  for (int j = 0; j < CFG.R - CFG.J; ++j) {  // the stored Cartesian rows
     double v = 0.0;
     if (cart && j < CFG.Cin) v = (double)cart[((size_t)b * CFG.Cin + j) * n0max + i];
     dst[CFG.J + j] = v;
@@ -556,6 +556,7 @@ __global__ void k_adjust_inc(WSP, int npts, int nb) {
   if (s.sWeights[1] + s.sWeights[2] < 1e-8) return;
   if (i >= s.nPts - 1) return;
   const int J = CFG.J;
+  const bool cartStored = w.R > J;  // otherwise the Cartesian rows are zeros (DevCfg::R)
   const size_t pst = (size_t)w.B * w.R;
   const double *p0 = w.P + (size_t)b * w.R + (size_t)i * pst, *nx = p0 + pst;
   double dthetaSQ = 0;
@@ -565,7 +566,7 @@ __global__ void k_adjust_inc(WSP, int npts, int nb) {
   }
   double dcartSQ = 0;
   for (int j = 0; j < 3; ++j) {
-    const double d = nx[J + j] - p0[J + j];
+    const double d = cartStored ? nx[J + j] - p0[J + j] : 0.0 - 0.0;
     dcartSQ += d * d;
   }
   double *o = w.nrm + ((size_t)(i + 1) * w.B + b) * 2;
@@ -597,12 +598,13 @@ __global__ void k_adjust_s(WSP, int special, int haveInc) {
   // haveInc: the increments sqrt(dthetaSQ), sqrt(dcartSQ) of point i+1 were left in its slots by k_adjust_inc (small
   // chunks: the pass is bound by the latency of one trajectory); otherwise they are formed here (full chunks: one
   // pass over the points instead of two)
+  const bool cartStored = w.R > J;  // otherwise the Cartesian rows are zeros (DevCfg::R)
   const size_t pst = (size_t)w.B * w.R;
   const double *p0 = w.P + (size_t)b * w.R;
   double cur[MAXD + 3];
   if (!haveInc) {
     for (int j = 0; j < J; ++j) cur[j] = p0[j];
-    for (int j = 0; j < 3; ++j) cur[MAXD + j] = p0[J + j];
+    for (int j = 0; j < 3; ++j) cur[MAXD + j] = cartStored ? p0[J + j] : 0.0;
   }
   // one point of the two running sums (+ the window bookkeeping of the automatic integration resolution)
   auto add_point = [&](int i, double it, double ic) {
@@ -646,7 +648,7 @@ __global__ void k_adjust_s(WSP, int special, int haveInc) {
       }
       double dcartSQ = 0;
       for (int j = 0; j < 3; ++j) {
-        const double v = nx[J + j];
+        const double v = cartStored ? nx[J + j] : 0.0;
         const double d = v - cur[MAXD + j];
         dcartSQ += d * d;
         cur[MAXD + j] = v;
@@ -767,15 +769,16 @@ __global__ void k_thomas_rows(WSP, double *src, double *dst, int nb, int b0, int
 // ba.cpp:651-781: constant-ds march along the weighted arc length.  Source rows P (+M), emits Q.
 // evalSplinePartials (ba.cpp:1341-1380) supplies the values; the Cartesian rows are refreshed
 // only when a Cartesian constraint is on, otherwise Traj::cartpt keeps its previous content.
-// JT / CT: joints and Cartesian rows as compile-time constants (0 = take them from the configuration), so that
-// the joint loops unroll and `last` / `cartpt` stay in registers instead of local memory.
+// JT / CT: joints and stored Cartesian rows as compile-time constants (JT = 0: both from the configuration), so
+// that the joint loops unroll and `last` / `cartpt` stay in registers instead of local memory.  CT = 0: the
+// Cartesian rows of a joint-only generic robot are not stored, their knots are read as a literal 0.0.
 template <int JT, int CT>
 __global__ void k_march(WSP) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= w.B) return;
   TrajState &s = w.st[b];
   if (s.status & ST_FATAL_MASK) return;
-  const int J = JT ? JT : CFG.J, C = CT ? CT : CFG.C, R = J + C;
+  const int J = JT ? JT : CFG.J, C = JT ? CT : w.R - J, R = J + C;
   const int nPts = s.nPts;
   const RV sC = vecv(w.sC, w, b);
   const size_t pst = (size_t)w.B * w.R;
@@ -788,7 +791,7 @@ __global__ void k_march(WSP) {
   #pragma unroll
   for (int j = 0; j < J; ++j) last[j] = P[j];
   #pragma unroll
-  for (int j = 0; j < 3; ++j) last[MAXD + j] = P[J + j];
+  for (int j = 0; j < 3; ++j) last[MAXD + j] = C ? P[J + j] : 0.0;
   double sPrv = 0, prv_ds = 0;
   int CurNewPt = 1, CurOldPt = 1;
   int seg = 0;
@@ -810,7 +813,7 @@ __global__ void k_march(WSP) {
     double dcartSQ = 0;
     #pragma unroll
     for (int j = 0; j < 3; ++j) {
-      const double d = po[J + j] - last[MAXD + j];
+      const double d = (C ? po[J + j] : 0.0) - last[MAXD + j];
       dcartSQ += d * d;
     }
     const double cur_ds = s.tTeachFact * s.sResi * (double)CurOldPt + s.thetaNormFact * sqrt(dthetaSQ) +
@@ -925,7 +928,8 @@ __global__ void k_march_group(WSP) {
   if (b >= w.B) return;  // (a whole group leaves together)
   TrajState &s = w.st[b];
   if (s.status & ST_FATAL_MASK) return;
-  const int J = CFG.J, C = CFG.C, R = J + C;
+  // C: the stored Cartesian rows; a joint-only generic robot stores none and reads rows J..J+2 as a literal 0.0
+  const int J = CFG.J, C = w.R - J, R = J + C;
   const bool isJ = r < J, isC = r >= J && r < R, isC3 = r >= J && r < J + 3, isCp = r >= J && r - J < MAXD;
   const int nPts = s.nPts;
   const RV sC = vecv(w.sC, w, b);
@@ -934,7 +938,7 @@ __global__ void k_march_group(WSP) {
   double *Q = w.Q + (size_t)b * w.R;
   const int Nc = w.Nc;
   if (r < R) Q[r] = P[r];
-  double last = (isJ || isC3) ? P[r] : 0.0;  // the previously emitted point: theta rows, cart xyz
+  double last = (isJ || (isC3 && C)) ? P[r] : 0.0;  // the previously emitted point: theta rows, cart xyz
   double cartpt = isCp ? s.cartpt[r - J] : 0.0;
   double sPrv = 0, prv_ds = 0;
   int CurNewPt = 1, CurOldPt = 1;
@@ -949,7 +953,7 @@ __global__ void k_march_group(WSP) {
     const double *po = P + (size_t)CurOldPt * pst;
     double dsq = 0.0;
     if (isJ || isC3) {
-      const double d = po[r] - last;
+      const double d = (isJ || C ? po[r] : 0.0) - last;
       dsq = d * d;
     }
     double dthetaSQ = 0;

@@ -195,6 +195,17 @@ Pmat make_pmat() {
 
 // ----------------------------------------------------------------------------- context
 #define NSETS 4
+// The shapes the two device workspaces are allocated for.  A shape holds every input of its array list (chunk_arrays,
+// out_arrays), so a held workspace serves a request when its shape covers the request's (ws_covers, out_covers).
+// B = 0 / Bo = 0: nothing held.
+struct WsShape {  // chunk-resident arrays; J..trq: the configuration's rows, which also size the output arrays
+  int B = 0, Nc = 0, Sc = 0, J = 0, Cin = 0, C = 0, R = 0, RT = 0;
+  bool trq = false;
+};
+struct OutShape {  // output sub-chunk arrays (rows as in the chunk's shape: ensure_ws drops these arrays with its own)
+  int Bo = 0, Sc = 0, Oc = 0, Os = 0, OutC = 0, rowP = 0, histP = 0;
+  bool keepF64 = false, fused = false;
+};
 struct batotp_ctx {
   int device = 0;
   cudaStream_t stream = 0;
@@ -204,17 +215,16 @@ struct batotp_ctx {
   DevCfg cfg;
   bool haveCfg = false;
   Ws w;
-  int capB = 0, capNc = 0, capSc = 0, capR = 0, capC = 0, capRT = 0;
-  bool capTrq = false;
+  WsShape wsHeld;
+  OutShape outHeld;
   std::vector<void *> wsAllocs;   // chunk-resident arrays
   size_t wsBytes = 0, outBytes = 0;  // bytes held by wsAllocs / outAllocs
   int learnedChunk = 0;              // automatic chunking: the chunk size the last batch call of this configuration ended with
-  int capBo = 0, capOc = 0, capOs = 0, capOutC = 0, capOSc = 0;
   std::vector<void *> outAllocs;  // output sub-chunk arrays
   int outChunk = 8192;            // trajectories per output pass
   // row pitch (points) of the packed float32 rows / histories: the caller's out_cap / hist_cap inside
   // batotp_cuda_optimize_batch (a sub-chunk then leaves in one contiguous copy), 0 = the device capacities
-  int rowPitch = 0, histPitch = 0, capRowPitch = 0, capHistPitch = 0;
+  int rowPitch = 0, histPitch = 0;
   // ragged result layout (batotp_batch_out.row_offset): the blocks of a sub-chunk are packed back to back in the
   // staging set and leave in one copy; where they go in the caller's buffer comes from a counter shared by the
   // contexts that work on one batch
@@ -272,10 +282,7 @@ struct batotp_ctx {
   cudaStream_t copyStream = 0;
   double *d_cartOutD = nullptr;
   double *d_outD = nullptr;  // [Bo][J+C+J][OutC] FP64 final rows (keepF64)
-  double *o_sOut = nullptr, *o_tauO = nullptr, *o_O5 = nullptr, *o_OA = nullptr, *o_OM = nullptr;
-  double *o_OD = nullptr, *o_OD2 = nullptr, *o_Trq = nullptr, *o_Trq2 = nullptr, *o_TrqM = nullptr;
-  int *o_segO = nullptr;
-  bool keepF64 = false, capKeep = false, capFused = false;
+  bool keepF64 = false;
   int mxSteps = 0;  // largest nFwd/nRev of the resident chunk (launch extents of the output phase)
   int allocPhase = 0;  // which workspace was being (re)allocated last: 0 chunk arrays, 1 output sub-chunk arrays
   // which buffers hold the final rows after interp_output
@@ -410,30 +417,28 @@ void free_ws(batotp_ctx *h) {
   for (void *p : h->wsAllocs) g_free(p);
   h->wsAllocs.clear();
   h->wsBytes = 0;
-  h->capB = 0;
+  h->wsHeld = WsShape();
 }
 void free_out(batotp_ctx *h) {
   for (void *p : h->outAllocs) g_free(p);
   h->outAllocs.clear();
   h->outBytes = 0;
-  h->capBo = 0;
-  h->capRowPitch = h->capHistPitch = 0;
+  h->outHeld = OutShape();
 }
 
-template <class T>
-T *ws_alloc(batotp_ctx *h, size_t count) {
-  void *p = g_alloc(count * sizeof(T));
-  h->wsAllocs.push_back(p);
-  h->wsBytes += count * sizeof(T);
-  return (T *)p;
-}
-template <class T>
-T *out_alloc(batotp_ctx *h, size_t count) {
-  void *p = g_alloc(count * sizeof(T));
-  h->outAllocs.push_back(p);
-  h->outBytes += count * sizeof(T);
-  return (T *)p;
-}
+// allocating visitor of chunk_arrays / out_arrays (a count of 0 leaves the member null)
+struct Allocate {
+  std::vector<void *> &allocs;
+  size_t &bytes;
+  template <class T>
+  void operator()(T *&p, size_t count) {
+    p = nullptr;
+    if (count == 0) return;
+    p = (T *)g_alloc(count * sizeof(T));
+    allocs.push_back(p);
+    bytes += count * sizeof(T);
+  }
+};
 
 void ensure_tabs(batotp_ctx *h, int n) {
   if (n <= h->tabN) return;
@@ -523,107 +528,152 @@ int final_cap(const batotp_ctx *h, int Sc, int Os) {
   return std::max(std::max(n, 16), Os);
 }
 
-// bytes of chunk-resident workspace per trajectory (the arrays of ensure_ws)
-size_t chunk_bytes_per_traj(const DevCfg &c, int Nc, int Sc) {
-  const size_t n = (size_t)Nc, sc = (size_t)Sc;
-  size_t per = 3 * (size_t)c.R * n * 8 + n * 8 + 2 * n * 8 + n * (size_t)c.RT * 32 + 5 * sc * 8 + 2 * sc + sizeof(TrajState);
-  if (c.trqOn) per += 2 * (size_t)4 * c.J * n * 8 + 2 * (size_t)c.R * n * 8;
-  return per;
+// capacities of the output arrays for a step capacity Sc: oversampled, smoothed and final points
+struct OutCaps { int Oc, Os, OutC; };
+OutCaps out_caps(const batotp_ctx *h, int Sc) {
+  const int Oc = oversample_cap(h, Sc);
+  const int Os = (!h->cfg.trqOn && smooth_uniform_on(h)) ? (int)(Oc / h->cfg.c.out_smooth_fact) + 16 : Oc;
+  return {Oc, Os, final_cap(h, Sc, Os)};
 }
 
-// bytes of output sub-chunk workspace per trajectory (the arrays of ensure_out) for a step capacity Sc
-size_t out_bytes_per_traj(const batotp_ctx *h, int Sc) {
+// The chunk-resident arrays (input phase + sweeps) of a workspace shaped s, as f(Ws member, element count).
+template <class F>
+void chunk_arrays(Ws &w, const WsShape &s, F &&f) {
+  const size_t b = (size_t)s.B, n = (size_t)s.Nc, sc = (size_t)s.Sc, R = (size_t)s.R;
+  f(w.P, b * R * n);
+  f(w.Q, b * R * n);
+  f(w.M, b * R * n);
+  f(w.sC, b * n);
+  f(w.nrm, b * 2 * n);
+  f(w.tab, b * n * s.RT * 4);
+  f(w.hist, b * 4 * sc);
+  f(w.flags, b * 2 * sc);
+  f(w.st, b);
+  f(w.mS, b * sc);
+  const size_t t = s.trq ? b : 0;  // torque only
+  f(w.A, t * 4 * s.J * n);
+  f(w.AM, t * 4 * s.J * n);
+  f(w.GD, t * R * n);
+  f(w.GD2, t * R * n);
+  f(w.queue, 4);
+  f(w.ragOff, b + 1);
+}
+
+// The output sub-chunk arrays of a workspace shaped s, as f(member, element count); a count of 0: not used.
+template <class F>
+void out_arrays(batotp_ctx *h, const OutShape &s, F &&f) {
   const DevCfg &c = h->cfg;
-  const size_t Oc = (size_t)oversample_cap(h, Sc);
-  const bool trq = c.trqOn != 0;
-  size_t Os = Oc;
-  if (!trq && smooth_uniform_on(h)) Os = (size_t)(Oc / c.c.out_smooth_fact) + 16;
-  const size_t OutC = (size_t)final_cap(h, Sc, (int)Os), R = (size_t)c.R;
-  size_t per = Oc * 20 + (fused_out(h) ? 0 : R * Oc * 8) + 2 * R * Os * 8;
-  if (trq) per += 2 * R * Oc * 8 + 3 * (size_t)MAXD * Oc * 8;
-  per += 2 * ((size_t)c.J * OutC * 4 + (size_t)std::max(c.Cin, 1) * OutC * 4 + (trq ? (size_t)c.J * OutC * 4 : 0) +
-              4 * (size_t)Sc * 4);
-  if (c.C == 7) per += 7 * OutC * 8;
-  if (h->keepF64) per += (size_t)(c.J + c.C + c.J) * OutC * 8;
-  return per;
+  Ws &w = h->w;
+  const size_t b = (size_t)s.Bo, R = (size_t)c.R, Oc = (size_t)s.Oc, Os = (size_t)s.Os, OutC = (size_t)s.OutC;
+  const size_t t = c.trqOn ? b : 0;  // torque only
+  f(w.sOut, b * Oc);
+  f(w.segO, b * Oc);
+  f(w.tauO, b * Oc);
+  f(w.O5, s.fused ? 8 : b * R * Oc);  // untouched on the fused path
+  f(w.OA, b * R * Os);
+  f(w.OM, b * R * Os);
+  f(w.OD, t * R * Oc);
+  f(w.OD2, t * R * Oc);
+  f(w.Trq, t * MAXD * Oc);
+  f(w.Trq2, t * MAXD * Oc);
+  f(w.TrqM, t * MAXD * Oc);
+  for (int q = 0; q < NSETS; ++q) {
+    f(h->o_thetaOut[q], b * c.J * s.rowP);
+    f(h->o_cartOut[q], b * std::max(c.Cin, 1) * s.rowP);
+    f(h->o_trqOut[q], t * c.J * s.rowP);
+    f(h->o_histOut[q], b * 4 * s.histP);
+  }
+  f(h->d_cartOutD, c.C == 7 ? b * 7 * OutC : 0);
+  f(h->d_outD, s.keepF64 ? b * (c.J + c.C + c.J) * OutC : 0);  // k_out_pack's layout
+}
+
+// (with a step hint the step capacity asked for is taken literally, not "at least")
+bool ws_covers(const WsShape &held, const WsShape &n, bool exactSc) {
+  return n.B <= held.B && n.Nc <= held.Nc && (exactSc ? n.Sc == held.Sc : n.Sc <= held.Sc) && n.J == held.J &&
+         n.Cin == held.Cin && n.C == held.C && n.R == held.R && n.RT == held.RT && n.trq == held.trq;
+}
+// the output arrays of a sub-chunk of Bo trajectories of a chunk with step capacity Sc, at the pitches in use
+OutShape out_shape(const batotp_ctx *h, int Bo, int Sc, int minOutC = 0) {
+  const OutCaps k = out_caps(h, Sc);
+  const int OutC = std::max(k.OutC, minOutC);
+  return {Bo, Sc, k.Oc, k.Os, OutC, h->rowPitch > 0 ? h->rowPitch : OutC, h->histPitch > 0 ? h->histPitch : Sc,
+          h->keepF64, fused_out(h)};
+}
+// (the output arrays belong to one step capacity of the chunk)
+bool out_covers(const OutShape &held, const OutShape &n) {
+  return n.Bo <= held.Bo && n.Sc == held.Sc && n.Oc <= held.Oc && n.Os <= held.Os && n.OutC <= held.OutC &&
+         n.rowP <= held.rowP && n.histP <= held.histP && n.keepF64 == held.keepF64 && n.fused == held.fused;
+}
+
+// The planner's footprints of a chunk shaped s: its arrays, the part of them that grows with each trajectory, and the
+// output arrays of its first sub-chunk.  They are the lists of arrays themselves, summed.
+struct Footprints { size_t chunk, perTraj, out; };
+Footprints footprints(batotp_ctx *h, const WsShape &s) {
+  size_t n = 0;
+  auto add = [&n](auto *&p, size_t count) { n += count * sizeof(*p); };
+  auto chunk_bytes = [&](int B) {
+    WsShape sb = s;
+    sb.B = B;
+    n = 0;
+    chunk_arrays(h->w, sb, add);
+    return n;
+  };
+  const size_t chunk = chunk_bytes(s.B), perTraj = chunk_bytes(1) - chunk_bytes(0);
+  n = 0;
+  out_arrays(h, out_shape(h, std::min(s.B, h->outChunk), s.Sc), add);
+  return {chunk, perTraj, n};
+}
+
+// A chunk whose arrays would not fit is refused before anything is freed or allocated, with the size that would fit
+// (the batch call continues with smaller chunks - and finds the workspace of its previous call intact: releasing and
+// re-allocating ~130 GB costs 170 ms).  Beside the chunk arrays the context will ask for the output arrays of one
+// sub-chunk and some slack for the input staging sets / the tail helper.
+void plan_chunk(batotp_ctx *h, const WsShape &want) {
+#ifndef BATOTP_HOST_EMU
+  const size_t held = h->wsBytes + h->outBytes;  // released if the new workspace goes ahead
+#else
+  const size_t held = 0;  // (BATOTP_EMU_FREE_MB is what this context may use in total)
+#endif
+  const Footprints fp = footprints(h, want);
+  const size_t fr = g_free_bytes() + held;
+  const size_t reserve = ((size_t)2 << 30) + fp.out;
+  const double room = (double)(fr > reserve ? fr - reserve : 0);
+  if ((double)fp.chunk > 0.94 * room) {
+    char buf[200];
+    snprintf(buf, sizeof buf, "chunk of %d trajectories needs %.1f GB of workspace (%zu bytes each), %.1f GB free",
+             want.B, (double)fp.chunk * 1e-9, fp.perTraj, (double)fr * 1e-9);
+    Err er{buf};
+    er.oom = true;
+    er.fitB = (int)std::min<double>(2.0e9, 0.9 * room / (double)fp.perTraj);
+    er.planned = true;
+    throw er;
+  }
 }
 
 // chunk-resident arrays (input phase + sweeps)
 void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
   const DevCfg &c = h->cfg;
-  const bool trq = c.trqOn != 0;
-  // (with a step hint the capacity asked for is taken literally, not "at least")
-  const bool scOk = h->stepHint > 0 ? (Sc == h->capSc) : (Sc <= h->capSc);
-  if (B <= h->capB && Nc <= h->capNc && scOk && c.R == h->capR && c.C == h->capC && c.RT == h->capRT &&
-      trq == h->capTrq && c.J == h->w.AD) {
+  const WsShape want{B, Nc, Sc, c.J, c.Cin, c.C, c.R, c.RT, c.trqOn != 0};
+  if (ws_covers(h->wsHeld, want, h->stepHint > 0)) {
     h->w.B = B;
     return;
   }
   h->allocPhase = 0;
-  {
-    // footprint of one trajectory in the chunk-resident arrays below; a chunk that cannot fit is refused before
-    // anything is freed or allocated, with the size that would fit (the batch call continues with smaller chunks -
-    // and finds the workspace of its previous call intact: releasing and re-allocating ~130 GB costs 170 ms)
-#ifndef BATOTP_HOST_EMU
-    const size_t held = h->wsBytes + h->outBytes;  // released below if the new workspace goes ahead
-#else
-    const size_t held = 0;  // (BATOTP_EMU_FREE_MB is what this context may use in total)
-#endif
-    const size_t per = chunk_bytes_per_traj(c, Nc, Sc);
-    const size_t fr = g_free_bytes() + held;
-    // what else this context will ask for: the output sub-chunk arrays (ensure_out) and some slack for the
-    // staging sets / the tail helper
-    const size_t reserve = ((size_t)2 << 30) + out_bytes_per_traj(h, Sc) * (size_t)std::min(B, h->outChunk);
-    if ((double)per * B > 0.94 * (double)(fr > reserve ? fr - reserve : 0)) {
-      char buf[200];
-      snprintf(buf, sizeof buf, "chunk of %d trajectories needs %.1f GB of workspace (%zu bytes each), %.1f GB free", B,
-               (double)per * B * 1e-9, per, (double)fr * 1e-9);
-      Err er{buf};
-      er.oom = true;
-      er.fitB = (int)std::min<double>(2.0e9, 0.9 * (double)(fr > reserve ? fr - reserve : 0) / (double)per);
-      er.planned = true;
-      throw er;
-    }
-  }
+  plan_chunk(h, want);
   free_ws(h);
   free_out(h);
   Ws &w = h->w;
   memset(&w, 0, sizeof(w));
   w.cfg = h->cfg;
-  const size_t b = (size_t)B;
-  const int R = c.R, RT = c.RT;
   w.B = B;
   w.Nc = Nc;
   w.Sc = Sc;
-  w.R = R;
-  w.RT = RT;
-  w.AD = c.J;
-  w.P = ws_alloc<double>(h, b * R * Nc);
-  w.Q = ws_alloc<double>(h, b * R * Nc);
-  w.M = ws_alloc<double>(h, b * R * Nc);
-  w.sC = ws_alloc<double>(h, b * Nc);
-  w.nrm = ws_alloc<double>(h, b * 2 * Nc);
-  w.tab = ws_alloc<double>(h, b * Nc * RT * 4);
-  w.hist = ws_alloc<double>(h, b * 4 * Sc);
-  w.flags = ws_alloc<unsigned char>(h, b * 2 * Sc);
-  w.st = ws_alloc<TrajState>(h, b);
-  w.mS = ws_alloc<double>(h, b * Sc);
-  if (trq) {
-    w.A = ws_alloc<double>(h, b * 4 * w.AD * Nc);
-    w.AM = ws_alloc<double>(h, b * 4 * w.AD * Nc);
-    w.GD = ws_alloc<double>(h, b * R * Nc);
-    w.GD2 = ws_alloc<double>(h, b * R * Nc);
-    g_zero(w.A, b * 4 * w.AD * Nc * sizeof(double), h->stream);
-  }
-  w.queue = ws_alloc<int>(h, 4);
-  w.ragOff = ws_alloc<long long>(h, b + 1);
-  h->capB = B;
-  h->capNc = Nc;
-  h->capSc = Sc;
-  h->capR = R;
-  h->capC = c.C;
-  h->capRT = RT;
-  h->capTrq = trq;
+  w.R = want.R;
+  w.RT = want.RT;
+  w.AD = want.J;
+  chunk_arrays(w, want, Allocate{h->wsAllocs, h->wsBytes});
+  if (want.trq) g_zero(w.A, (size_t)B * 4 * w.AD * Nc * sizeof(double), h->stream);
+  h->wsHeld = want;
   ensure_tabs(h, std::max(Nc, Sc) + 8);
 }
 
@@ -640,71 +690,19 @@ void select_out_set(batotp_ctx *h, int q) {
 
 // output sub-chunk arrays, sized from the step capacity of the resident chunk
 void ensure_out(batotp_ctx *h, int Bo, int minOutC = 0) {
-  const DevCfg &c = h->cfg;
   Ws &w = h->w;
-  const int Sc = w.Sc;
-  const int Oc = oversample_cap(h, Sc);
-  const bool trq = c.trqOn != 0;
-  int Os = Oc;
-  if (!trq && smooth_uniform_on(h)) Os = (int)(Oc / c.c.out_smooth_fact) + 16;
-  const int OutC = std::max(final_cap(h, Sc, Os), minOutC);
-  const int rowP = h->rowPitch > 0 ? h->rowPitch : OutC, histP = h->histPitch > 0 ? h->histPitch : Sc;
-  if (!(Bo <= h->capBo && Oc <= h->capOc && Os <= h->capOs && OutC <= h->capOutC && Sc == h->capOSc &&
-        rowP <= h->capRowPitch && histP <= h->capHistPitch &&
-        h->keepF64 == h->capKeep && fused_out(h) == h->capFused && c.R == h->capR && trq == h->capTrq)) {
-    free_out(h);
-    h->allocPhase = 1;
-    const size_t b = (size_t)Bo;
-    const int R = c.R;
-    h->o_sOut = out_alloc<double>(h, b * Oc);
-    h->o_segO = out_alloc<int>(h, b * Oc);
-    h->o_tauO = out_alloc<double>(h, b * Oc);
-    h->o_O5 = out_alloc<double>(h, fused_out(h) ? 8 : b * R * Oc);  // untouched on the fused path
-    h->o_OA = out_alloc<double>(h, b * R * Os);
-    h->o_OM = out_alloc<double>(h, b * R * Os);
-    h->o_OD = h->o_OD2 = h->o_Trq = h->o_Trq2 = h->o_TrqM = nullptr;
-    if (trq) {
-      h->o_OD = out_alloc<double>(h, b * R * Oc);
-      h->o_OD2 = out_alloc<double>(h, b * R * Oc);
-      h->o_Trq = out_alloc<double>(h, b * MAXD * Oc);
-      h->o_Trq2 = out_alloc<double>(h, b * MAXD * Oc);
-      h->o_TrqM = out_alloc<double>(h, b * MAXD * Oc);
-    }
-    for (int q = 0; q < NSETS; ++q) {
-      h->setBusy[q] = false;  // (free_out has waited for the device)
-      h->o_thetaOut[q] = out_alloc<float>(h, b * c.J * rowP);
-      h->o_cartOut[q] = out_alloc<float>(h, b * std::max(c.Cin, 1) * rowP);
-      h->o_trqOut[q] = trq ? out_alloc<float>(h, b * c.J * rowP) : nullptr;
-      h->o_histOut[q] = out_alloc<float>(h, b * 4 * histP);
-    }
-    h->capRowPitch = rowP;
-    h->capHistPitch = histP;
-    select_out_set(h, 0);
-    h->d_cartOutD = (c.C == 7) ? out_alloc<double>(h, b * 7 * OutC) : nullptr;
-    h->d_outD = h->keepF64 ? out_alloc<double>(h, b * (c.J + c.C + c.J) * OutC) : nullptr;  // k_out_pack's layout
-    h->capBo = Bo;
-    h->capOc = Oc;
-    h->capOs = Os;
-    h->capOutC = OutC;
-    h->capOSc = Sc;
-    h->capKeep = h->keepF64;
-    h->capFused = fused_out(h);
-    ensure_tabs(h, std::max(std::max(w.Nc, Sc), Oc) + 8);
-  }
-  w.Oc = h->capOc;
-  w.Os = h->capOs;
-  w.OutC = h->capOutC;
-  w.sOut = h->o_sOut;
-  w.segO = h->o_segO;
-  w.tauO = h->o_tauO;
-  w.O5 = h->o_O5;
-  w.OA = h->o_OA;
-  w.OM = h->o_OM;
-  w.OD = h->o_OD;
-  w.OD2 = h->o_OD2;
-  w.Trq = h->o_Trq;
-  w.Trq2 = h->o_Trq2;
-  w.TrqM = h->o_TrqM;
+  const OutShape want = out_shape(h, Bo, w.Sc, minOutC);
+  if (out_covers(h->outHeld, want)) return;
+  free_out(h);
+  h->allocPhase = 1;
+  out_arrays(h, want, Allocate{h->outAllocs, h->outBytes});
+  h->outHeld = want;
+  for (bool &busy : h->setBusy) busy = false;  // (free_out has waited for the device)
+  select_out_set(h, 0);
+  w.Oc = want.Oc;
+  w.Os = want.Os;
+  w.OutC = want.OutC;
+  ensure_tabs(h, std::max(std::max(w.Nc, w.Sc), want.Oc) + 8);
 }
 
 void set_cfg(batotp_ctx *h, const batotp_cfg *cfg) {
@@ -1290,9 +1288,10 @@ void do_interp_output(batotp_ctx *h, int b0, int Bo) {
   w.b0 = b0;
   w.Bo = Bo;
   const ThomasTabs t = thomas_tabs(h);
-  // launch extents from the longest trajectory of the chunk rather than from the capacities
-  const int lOc = std::min(w.Oc, oversample_cap(h, std::max(h->mxSteps, 4)));
-  const int lOs = (w.Os == w.Oc) ? lOc : std::min(w.Os, (int)(lOc / c.c.out_smooth_fact) + 16);
+  // launch extents from the longest trajectory of the chunk rather than from the capacities (held Os == Oc: no
+  // smoothing, or capacities too small for it to shrink them - the smoothed rows then span the oversampled extent)
+  const OutCaps l = out_caps(h, std::max(h->mxSteps, 4));
+  const int lOc = std::min(w.Oc, l.Oc), lOs = (w.Os == w.Oc) ? lOc : std::min(w.Os, l.Os);
   // s(t) of the whole resident chunk is planned with its first sub-chunk: one launch of the sequential solve over
   // the chunk's trajectories instead of one per sub-chunk (mS is chunk-resident, [B][Sc])
   if (b0 == 0) LAUNCH_T(h, k_out_plan, h->B, w, t);
@@ -1839,6 +1838,16 @@ int batotp_emu_set_rcp_ulps(int k) {
   g_emu_rcp_ulps = k;
   return 0;
 }
+// TEST-ONLY: the planner's footprints of the chunk workspace the context holds - its chunk arrays, the output arrays
+// of its first sub-chunk, the bytes per trajectory - beside the bytes actually held and the trajectories the chunk
+// arrays were allocated for: {chunk, out, perTraj, wsBytes, outBytes, B}
+int batotp_emu_workspace_plan(batotp_handle h, size_t *out) {
+  if (!h || !out) return -1;
+  const Footprints fp = footprints(h, h->wsHeld);
+  const size_t v[6] = {fp.chunk, fp.out, fp.perTraj, h->wsBytes, h->outBytes, (size_t)h->wsHeld.B};
+  memcpy(out, v, sizeof v);
+  return 0;
+}
 #endif
 int batotp_cuda_selftest_bisect(batotp_handle h, unsigned long long seed, long long n, long long *mismatches) {
   if (!h || n < 0) return -1;
@@ -2342,7 +2351,7 @@ static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batc
     const double tC0 = g_trace() ? g_now_ms() : 0;
     if (g_trace())
       fprintf(stderr, "[batotp] chunk at %d: %d paths (chunk setting %d, round capacity %d; capB %d capNc %d capSc %d; alloc %.1f ms free %.1f ms so far)\n",
-              at, B, chunk, sweep_round_capacity(h, cfg, B), h->capB, h->capNc, h->capSc, g_allocMs, g_freeMs);
+              at, B, chunk, sweep_round_capacity(h, cfg, B), h->wsHeld.B, h->wsHeld.Nc, h->wsHeld.Sc, g_allocMs, g_freeMs);
     try {
       process_chunk(h, first ? cfg : nullptr, in, out, at, B, nextB);
     } catch (const Err &e) {

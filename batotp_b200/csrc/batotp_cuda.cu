@@ -206,11 +206,38 @@ struct OutShape {  // output sub-chunk arrays (rows as in the chunk's shape: ens
   int Bo = 0, Sc = 0, Oc = 0, Os = 0, OutC = 0, rowP = 0, histP = 0;
   bool keepF64 = false, fused = false;
 };
+// The caller's options (batotp_cuda_set_*).  The tail helper of a batch call runs under a copy of them.
+struct Settings {
+  int chunk = 0;         // trajectories per resident chunk; 0 = automatic (auto_chunk)
+  int outChunk = 8192;   // trajectories per output pass
+  int maxSteps = 65536;  // largest RK-step capacity the automatic retries grow to (per sweep)
+  int stepHint = 0;      // RK-step capacity a chunk starts with (0 = automatic: max(1024, 2 x grid points))
+  int sweepKernel = 0;   // 0 automatic (by chunk size), 1 one trajectory per lane (k_sweep), 2 a group of lanes per trajectory (k_sweep_group)
+  int walkerKernel = 0;  // sequential walkers of the input phase (cumulative norms, interpSpecial march): 0 by chunk size, 1 one thread per trajectory, 2 point-parallel increments + a group of lanes per trajectory
+  // tail overlap (batotp_cuda_optimize_batch): a last chunk that fills at most one sweep CTA per SM runs on a second
+  // context (own streams and workspaces, one host thread) next to the output / input phases of the full chunks
+  bool tailOverlap = true;
+  bool keepF64 = false;  // FP64 side output of the final rows (d_outD)
+  bool profile = false;  // per-kernel device timing (batotp_cuda_set_profile): serialises every launch
+  // cfg.dyn_source = 1: the caller's point function for a1..a4 (Robot::call_dynSerial's contract)
+  batotp_dyn_fn dynFn = nullptr;
+  void *dynUser = nullptr;
+};
+// One staging set of packed float32 output rows.  The rows of sub-chunk k travel to the host on the copy stream while
+// the kernels of the following sub-chunks fill the other sets - and, since nothing but the output phase touches a set,
+// while the NEXT chunk's input phase and sweeps run: when the host link is the bottleneck (several GPUs sharing it)
+// the copy engine then never idles.
+struct OutSet {
+  float *theta = nullptr, *cart = nullptr, *trq = nullptr, *hist = nullptr;
+  bool busy = false;  // a copy out of the set has been enqueued since its rows were last awaited (copied)
+  long long ragBase = 0, ragTotal = 0;  // ragged layout: where the set's blocks go in the caller's buffers, their points
+  cudaEvent_t packed = {}, copied = {};  // the output phase has filled the set / its copy to the caller has completed
+};
 struct batotp_ctx {
   int device = 0;
   cudaStream_t stream = 0;
   std::string err;
-  int chunk = 0;  // trajectories per resident chunk; 0 = automatic (auto_chunk)
+  Settings opt;
   long launches = 0;
   DevCfg cfg;
   bool haveCfg = false;
@@ -221,25 +248,9 @@ struct batotp_ctx {
   size_t wsBytes = 0, outBytes = 0;  // bytes held by wsAllocs / outAllocs
   int learnedChunk = 0;              // automatic chunking: the chunk size the last batch call of this configuration ended with
   std::vector<void *> outAllocs;  // output sub-chunk arrays
-  int outChunk = 8192;            // trajectories per output pass
-  // row pitch (points) of the packed float32 rows / histories: the caller's out_cap / hist_cap inside
-  // batotp_cuda_optimize_batch (a sub-chunk then leaves in one contiguous copy), 0 = the device capacities
-  int rowPitch = 0, histPitch = 0;
-  // ragged result layout (batotp_batch_out.row_offset): the blocks of a sub-chunk are packed back to back in the
-  // staging set and leave in one copy; where they go in the caller's buffer comes from a counter shared by the
-  // contexts that work on one batch
-  bool ragged = false;
-  std::atomic<long long> *ragNext = nullptr;
+  // ragged result layout of the resident chunk (plan_ragged)
   std::vector<long long> ragOffHost;  // [B + 1] prefix sums of the resident chunk's output lengths (w.ragOff on the device)
   long long ragChunkBase = 0;         // where the chunk's blocks start in the caller's buffers
-  long long ragBase[NSETS] = {}, ragTotal[NSETS] = {};
-  int curSet = 0;
-  int maxSteps = 65536;           // largest RK-step capacity the automatic retries grow to (per sweep)
-  // cfg.dyn_source = 1: the caller's point function for a1..a4 (Robot::call_dynSerial's contract)
-  batotp_dyn_fn dynFn = nullptr;
-  void *dynUser = nullptr;
-  int sweepKernel = 0;            // 0 automatic (by chunk size), 1 one trajectory per lane (k_sweep), 2 a group of lanes per trajectory (k_sweep_group)
-  int stepHint = 0;               // RK-step capacity a chunk starts with (0 = automatic: max(1024, 2 x grid points))
   // Thomas factor tables
   double *d_cN = nullptr;  // Thomas tables (ensure_tabs)
   int tabN = 0;
@@ -271,18 +282,12 @@ struct batotp_ctx {
   bool inF64 = false, hasTheta = false, hasCart = false;
   int B = 0, n0max = 0;
   // staged outputs
-  float *d_thetaOut = nullptr, *d_cartOut = nullptr, *d_trqOut = nullptr, *d_histOut = nullptr;  // current set
-  // NSETS sets of packed-output staging buffers: the rows of sub-chunk k travel to the host on the copy stream
-  // while the kernels of the following sub-chunks fill the other sets - and, since nothing but the output phase
-  // touches a set, while the NEXT chunk's input phase and sweeps run: when the host link is the bottleneck (several
-  // GPUs sharing it) the copy engine then never idles
-  float *o_thetaOut[NSETS] = {}, *o_cartOut[NSETS] = {}, *o_trqOut[NSETS] = {}, *o_histOut[NSETS] = {};
-  bool setBusy[NSETS] = {};  // a copy out of the set has been enqueued since its rows were last awaited (evCopied)
-  int setNext = 0;           // the staging sets rotate across sub-chunks AND chunks
+  OutSet sets[NSETS];
+  OutSet *outSet = sets;  // the set the output phase packs into and the fetch copies from
+  int setNext = 0;        // the staging sets rotate across sub-chunks AND chunks
   cudaStream_t copyStream = 0;
   double *d_cartOutD = nullptr;
   double *d_outD = nullptr;  // [Bo][J+C+J][OutC] FP64 final rows (keepF64)
-  bool keepF64 = false;
   int mxSteps = 0;  // largest nFwd/nRev of the resident chunk (launch extents of the output phase)
   int allocPhase = 0;  // which workspace was being (re)allocated last: 0 chunk arrays, 1 output sub-chunk arrays
   // which buffers hold the final rows after interp_output
@@ -305,29 +310,44 @@ struct batotp_ctx {
   // learnt from the launches of the current configuration ([0] lane kernel, [1] group kernel; key = its dispatch key)
   int sweepCap[2] = {0, 0}, sweepCapKey = -1;
   long long cntVerify = 0, cntSteps = 0, cntTraj = 0;
-  // optional per-kernel device timing (batotp_cuda_set_profile): serialises every launch
-  bool profile = false;
-  std::map<std::string, std::pair<double, long>> prof;
-  // tail overlap (batotp_cuda_optimize_batch): a last chunk that fills at most one sweep CTA per SM runs on a second
-  // context (own streams and workspaces, one host thread) next to the output / input phases of the full chunks
-  batotp_ctx *helper = nullptr;
-  bool tailOverlap = true;
-  int walkerKernel = 0;  // sequential walkers of the input phase (cumulative norms, interpSpecial march): 0 by chunk size, 1 one thread per trajectory, 2 point-parallel increments + a group of lanes per trajectory
-  // stragglers: the few trajectories of a chunk that outgrow the step capacity keep BATOTP_ST_STEP_CAP for the
-  // moment and are re-run together, with a larger capacity, after the chunks of the batch (optimize_batch)
-  std::vector<int> stragglers;  // indices in the caller's batch
-  int stragglerSc = 0;          // the step capacity they outgrew
-  int chunkFirst = 0;           // index of the resident chunk's first trajectory in the caller's batch
-  bool collectStragglers = false;
-  std::function<void()> onSweepsDone;  // called once the sweeps of a chunk have completed on the device
-  std::function<void()> beforeSweeps;  // called after interpInputData of a chunk has been enqueued (may block)
+  std::map<std::string, std::pair<double, long>> prof;  // per-kernel device timing (opt.profile)
+  batotp_ctx *helper = nullptr;  // the second context of the tail overlap (opt.tailOverlap)
 #ifndef BATOTP_HOST_EMU
   cudaEvent_t evS0 = nullptr, evS1 = nullptr, evT[2] = {nullptr, nullptr}, evP[2] = {nullptr, nullptr};
-  cudaEvent_t evOut[NSETS] = {}, evCopied[NSETS] = {};
   bool sweepPending = false;
-#else
-  cudaEvent_t evOut[NSETS] = {}, evCopied[NSETS] = {};
 #endif
+};
+
+// The state of one batch call (batotp_cuda_optimize_batch): where its results go and how they are laid out, and the
+// trajectories it leaves for a second pass.  It lives on the caller's stack and is passed down; the phase-wise entry
+// points use a default run (rows at the device capacities, no ragged layout, nothing collected).
+struct BatchRun {
+  const batotp_cfg *cfg = nullptr;
+  const batotp_batch_in *in = nullptr;
+  batotp_batch_out *out = nullptr;
+  // row pitch (points) of the packed float32 rows / histories: the caller's out_cap / hist_cap (a sub-chunk then
+  // leaves in one contiguous copy), 0 = the device capacities
+  int rowPitch = 0, histPitch = 0;
+  // ragged result layout (batotp_batch_out.row_offset): the blocks of a sub-chunk are packed back to back in the
+  // staging set and leave in one copy; where they go in the caller's buffer comes from a counter shared by the
+  // contexts that work on one batch
+  bool ragged = false;
+  std::atomic<long long> *ragNext = nullptr;
+  // stragglers: the few trajectories of a chunk that outgrow the step capacity keep BATOTP_ST_STEP_CAP for the
+  // moment and are re-run together, with a larger capacity, after the chunks of the batch
+  bool collect = false;
+  std::vector<int> stragglers;  // indices in the caller's batch
+  int stragglerSc = 0;          // the step capacity they outgrew
+  std::function<void()> onSweepsDone;  // called once the sweeps of a chunk have completed on the device
+  std::function<void()> beforeSweeps;  // called after interpInputData of a chunk has been enqueued (may block)
+
+  BatchRun() = default;
+  // the results go to `out`; ragNext: the shared counter of a ragged layout (nullptr: the rows are pitched)
+  BatchRun(const batotp_cfg *c, const batotp_batch_in *i, batotp_batch_out *o, std::atomic<long long> *rag, bool coll)
+      : cfg(c), in(i), out(o), ragged(o->row_offset != nullptr && rag != nullptr), ragNext(rag), collect(coll) {
+    rowPitch = (!ragged && (o->theta_out || o->cart_out || o->trq_out) && o->out_cap > 0) ? o->out_cap : 0;
+    histPitch = (o->hist && o->hist_cap > 0) ? o->hist_cap : 0;
+  }
 };
 
 namespace {
@@ -338,7 +358,7 @@ struct ProfScope {
   const char *name;
   ProfScope(batotp_ctx *h_, const char *n) : h(h_), name(n) {
 #ifndef BATOTP_HOST_EMU
-    if (h->profile) {
+    if (h->opt.profile) {
       if (!h->evP[0]) {
         cudaEventCreate(&h->evP[0]);
         cudaEventCreate(&h->evP[1]);
@@ -349,7 +369,7 @@ struct ProfScope {
   }
   ~ProfScope() {
 #ifndef BATOTP_HOST_EMU
-    if (h->profile) {
+    if (h->opt.profile) {
       cudaEventRecord(h->evP[1], h->stream);
       cudaEventSynchronize(h->evP[1]);
       float ms = 0;
@@ -577,11 +597,11 @@ void out_arrays(batotp_ctx *h, const OutShape &s, F &&f) {
   f(w.Trq, t * MAXD * Oc);
   f(w.Trq2, t * MAXD * Oc);
   f(w.TrqM, t * MAXD * Oc);
-  for (int q = 0; q < NSETS; ++q) {
-    f(h->o_thetaOut[q], b * c.J * s.rowP);
-    f(h->o_cartOut[q], b * std::max(c.Cin, 1) * s.rowP);
-    f(h->o_trqOut[q], t * c.J * s.rowP);
-    f(h->o_histOut[q], b * 4 * s.histP);
+  for (OutSet &o : h->sets) {
+    f(o.theta, b * c.J * s.rowP);
+    f(o.cart, b * std::max(c.Cin, 1) * s.rowP);
+    f(o.trq, t * c.J * s.rowP);
+    f(o.hist, b * 4 * s.histP);
   }
   f(h->d_cartOutD, c.C == 7 ? b * 7 * OutC : 0);
   f(h->d_outD, s.keepF64 ? b * (c.J + c.C + c.J) * OutC : 0);  // k_out_pack's layout
@@ -592,12 +612,12 @@ bool ws_covers(const WsShape &held, const WsShape &n, bool exactSc) {
   return n.B <= held.B && n.Nc <= held.Nc && (exactSc ? n.Sc == held.Sc : n.Sc <= held.Sc) && n.J == held.J &&
          n.Cin == held.Cin && n.C == held.C && n.R == held.R && n.RT == held.RT && n.trq == held.trq;
 }
-// the output arrays of a sub-chunk of Bo trajectories of a chunk with step capacity Sc, at the pitches in use
-OutShape out_shape(const batotp_ctx *h, int Bo, int Sc, int minOutC = 0) {
+// the output arrays of a sub-chunk of Bo trajectories of a chunk with step capacity Sc, at the pitches of run r
+OutShape out_shape(const batotp_ctx *h, const BatchRun &r, int Bo, int Sc, int minOutC = 0) {
   const OutCaps k = out_caps(h, Sc);
   const int OutC = std::max(k.OutC, minOutC);
-  return {Bo, Sc, k.Oc, k.Os, OutC, h->rowPitch > 0 ? h->rowPitch : OutC, h->histPitch > 0 ? h->histPitch : Sc,
-          h->keepF64, fused_out(h)};
+  return {Bo, Sc, k.Oc, k.Os, OutC, r.rowPitch > 0 ? r.rowPitch : OutC, r.histPitch > 0 ? r.histPitch : Sc,
+          h->opt.keepF64, fused_out(h)};
 }
 // (the output arrays belong to one step capacity of the chunk)
 bool out_covers(const OutShape &held, const OutShape &n) {
@@ -608,7 +628,7 @@ bool out_covers(const OutShape &held, const OutShape &n) {
 // The planner's footprints of a chunk shaped s: its arrays, the part of them that grows with each trajectory, and the
 // output arrays of its first sub-chunk.  They are the lists of arrays themselves, summed.
 struct Footprints { size_t chunk, perTraj, out; };
-Footprints footprints(batotp_ctx *h, const WsShape &s) {
+Footprints footprints(batotp_ctx *h, const BatchRun &r, const WsShape &s) {
   size_t n = 0;
   auto add = [&n](auto *&p, size_t count) { n += count * sizeof(*p); };
   auto chunk_bytes = [&](int B) {
@@ -620,7 +640,7 @@ Footprints footprints(batotp_ctx *h, const WsShape &s) {
   };
   const size_t chunk = chunk_bytes(s.B), perTraj = chunk_bytes(1) - chunk_bytes(0);
   n = 0;
-  out_arrays(h, out_shape(h, std::min(s.B, h->outChunk), s.Sc), add);
+  out_arrays(h, out_shape(h, r, std::min(s.B, h->opt.outChunk), s.Sc), add);
   return {chunk, perTraj, n};
 }
 
@@ -628,13 +648,13 @@ Footprints footprints(batotp_ctx *h, const WsShape &s) {
 // (the batch call continues with smaller chunks - and finds the workspace of its previous call intact: releasing and
 // re-allocating ~130 GB costs 170 ms).  Beside the chunk arrays the context will ask for the output arrays of one
 // sub-chunk and some slack for the input staging sets / the tail helper.
-void plan_chunk(batotp_ctx *h, const WsShape &want) {
+void plan_chunk(batotp_ctx *h, const BatchRun &r, const WsShape &want) {
 #ifndef BATOTP_HOST_EMU
   const size_t held = h->wsBytes + h->outBytes;  // released if the new workspace goes ahead
 #else
   const size_t held = 0;  // (BATOTP_EMU_FREE_MB is what this context may use in total)
 #endif
-  const Footprints fp = footprints(h, want);
+  const Footprints fp = footprints(h, r, want);
   const size_t fr = g_free_bytes() + held;
   const size_t reserve = ((size_t)2 << 30) + fp.out;
   const double room = (double)(fr > reserve ? fr - reserve : 0);
@@ -651,15 +671,15 @@ void plan_chunk(batotp_ctx *h, const WsShape &want) {
 }
 
 // chunk-resident arrays (input phase + sweeps)
-void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
+void ensure_ws(batotp_ctx *h, const BatchRun &r, int B, int Nc, int Sc) {
   const DevCfg &c = h->cfg;
   const WsShape want{B, Nc, Sc, c.J, c.Cin, c.C, c.R, c.RT, c.trqOn != 0};
-  if (ws_covers(h->wsHeld, want, h->stepHint > 0)) {
+  if (ws_covers(h->wsHeld, want, h->opt.stepHint > 0)) {
     h->w.B = B;
     return;
   }
   h->allocPhase = 0;
-  plan_chunk(h, want);
+  plan_chunk(h, r, want);
   free_ws(h);
   free_out(h);
   Ws &w = h->w;
@@ -677,28 +697,20 @@ void ensure_ws(batotp_ctx *h, int B, int Nc, int Sc) {
   ensure_tabs(h, std::max(Nc, Sc) + 8);
 }
 
-inline int row_pitch(const batotp_ctx *h) { return h->rowPitch > 0 ? h->rowPitch : h->w.OutC; }
-inline int hist_pitch(const batotp_ctx *h) { return h->histPitch > 0 ? h->histPitch : h->w.Sc; }
-
-void select_out_set(batotp_ctx *h, int q) {
-  h->curSet = q;
-  h->d_thetaOut = h->o_thetaOut[q];
-  h->d_cartOut = h->o_cartOut[q];
-  h->d_trqOut = h->o_trqOut[q];
-  h->d_histOut = h->o_histOut[q];
-}
+inline int row_pitch(const batotp_ctx *h, const BatchRun &r) { return r.rowPitch > 0 ? r.rowPitch : h->w.OutC; }
+inline int hist_pitch(const batotp_ctx *h, const BatchRun &r) { return r.histPitch > 0 ? r.histPitch : h->w.Sc; }
 
 // output sub-chunk arrays, sized from the step capacity of the resident chunk
-void ensure_out(batotp_ctx *h, int Bo, int minOutC = 0) {
+void ensure_out(batotp_ctx *h, const BatchRun &r, int Bo, int minOutC = 0) {
   Ws &w = h->w;
-  const OutShape want = out_shape(h, Bo, w.Sc, minOutC);
+  const OutShape want = out_shape(h, r, Bo, w.Sc, minOutC);
   if (out_covers(h->outHeld, want)) return;
   free_out(h);
   h->allocPhase = 1;
   out_arrays(h, want, Allocate{h->outAllocs, h->outBytes});
   h->outHeld = want;
-  for (bool &busy : h->setBusy) busy = false;  // (free_out has waited for the device)
-  select_out_set(h, 0);
+  for (OutSet &o : h->sets) o.busy = false;  // (free_out has waited for the device)
+  h->outSet = h->sets;
   w.Oc = want.Oc;
   w.Os = want.Os;
   w.OutC = want.OutC;
@@ -767,7 +779,7 @@ int check_cfg(batotp_ctx *h) {
       h->err = "dyn_source = 1 (a caller-supplied dynamic model) serves serial mechanisms only";
       return -1;
     }
-    if (!h->dynFn) {
+    if (!h->opt.dynFn) {
       h->err = "dyn_source = 1 needs a point function: call batotp_cuda_set_dyn_callback first";
       return -1;
     }
@@ -974,7 +986,7 @@ int dispatch_sweep(batotp_ctx *h) {
     h->err = "parallel-mechanism torque limits without isPar2Ser are instantiated for 3 joints + Cartesian limits (CSPR3DOF)";
     return -1;
   }
-  const bool group = group_sweep(c, h->sweepKernel, h->B);
+  const bool group = group_sweep(c, h->opt.sweepKernel, h->B);
   switch (key) {
     case 7 * 4 + 0: launch_sweep<7, false, false>(h, group); return 0;  // GEN7DOF
     case 7 * 4 + 2: launch_sweep<7, true, false>(h, group); return 0;   // KUKA-LWR-IV
@@ -1150,7 +1162,7 @@ int do_interp_input(batotp_ctx *h, bool haveN0, bool planSync) {
     // chunks that do not fill the machine are bound by the latency of one trajectory in the one-thread-per-trajectory
     // walkers: their per-point work goes to point-parallel / group kernels (measured on the B200: KUKA x4096 march
     // 107 -> 24.5 ms, cumulative norms 23.5 -> 12.4 ms; GEN7DOF x56832 19.5 -> 22.6 and 2.2 -> 3.1 ms, hence the switch)
-    const bool smallChunk = h->walkerKernel == 2 || (h->walkerKernel == 0 && B <= WALKER_GROUP_MAX_B);
+    const bool smallChunk = h->opt.walkerKernel == 2 || (h->opt.walkerKernel == 0 && B <= WALKER_GROUP_MAX_B);
     if (smallChunk) LAUNCH_TP(h, k_adjust_inc, w.Nc, B, w);
     LAUNCH_T(h, k_adjust_s, B, w, 1, smallChunk ? 1 : 0);
     if (planSync) {
@@ -1222,11 +1234,11 @@ int do_interp_input(batotp_ctx *h, bool haveN0, bool planSync) {
 // BA::interpInputData with _isInterpOnly (ba.cpp:139-159) for the resident chunk: re-sample every row with
 // natural splines at outRes; the result is packed like an optimised trajectory (one output "sub-chunk" =
 // the whole chunk, whose point-major layout the packing kernel reads directly).
-int do_interp_only(batotp_ctx *h, bool haveN0) {
+int do_interp_only(batotp_ctx *h, const BatchRun &r, bool haveN0) {
   const DevCfg &c = h->cfg;
   for (int attempt = 0; attempt < 4; ++attempt) {
     int Nc = std::max(std::max(h->hwNc, h->n0max + 8), h->w.Nc);
-    ensure_ws(h, h->B, Nc, std::max(h->hwSc, 1024));
+    ensure_ws(h, r, h->B, Nc, std::max(h->hwSc, 1024));
     Ws &w = h->w;
     w.B = h->B;
     run_load_prepare(h, haveN0);
@@ -1255,18 +1267,19 @@ int do_interp_only(batotp_ctx *h, bool haveN0) {
     LAUNCH_TP(h, k_resample_check, w.Nc, h->B, w);
     LAUNCH_T(h, k_resample_commit, h->B, w);
     std::swap(w.P, w.Q);
-    ensure_out(h, h->B, mx + 8);
+    ensure_out(h, r, h->B, mx + 8);
     w.b0 = 0;
     w.Bo = h->B;
     LAUNCH_T(h, k_interp_only_finish, h->B, w);
-    select_out_set(h, 0);
+    h->outSet = h->sets;
+    const OutSet &o = h->sets[0];
     const bool strictQuat = (c.C == 7 && c.c.trig_mode != 0);
-    const int rp = row_pitch(h), hp = hist_pitch(h);
-    if (h->d_trqOut) g_zero(h->d_trqOut, (size_t)h->B * c.J * rp * sizeof(float), h->stream);  // no torque rows here
-    LAUNCH_PT(h, k_out_pack, std::max(w.OutC, rp), h->B, w, w.P, w.M, (double *)nullptr, (double *)nullptr, h->d_thetaOut,
-              h->d_cartOut, (float *)nullptr, strictQuat ? h->d_cartOutD : (double *)nullptr, h->d_outD, rp,
+    const int rp = row_pitch(h, r), hp = hist_pitch(h, r);
+    if (o.trq) g_zero(o.trq, (size_t)h->B * c.J * rp * sizeof(float), h->stream);  // no torque rows here
+    LAUNCH_PT(h, k_out_pack, std::max(w.OutC, rp), h->B, w, w.P, w.M, (double *)nullptr, (double *)nullptr, o.theta,
+              o.cart, (float *)nullptr, strictQuat ? h->d_cartOutD : (double *)nullptr, h->d_outD, rp,
               (const long long *)nullptr, 0ll);
-    LAUNCH_PT(h, k_pack_hist, std::max(w.Sc, hp), h->B, w, h->d_histOut, hp);
+    LAUNCH_PT(h, k_pack_hist, std::max(w.Sc, hp), h->B, w, o.hist, hp);
     h->phase = 4;
     return 0;
   }
@@ -1281,9 +1294,9 @@ int do_sweeps(batotp_ctx *h) {
 }
 
 // interpOutputData for the sub-chunk [b0, b0+Bo) of the resident chunk
-void do_interp_output(batotp_ctx *h, int b0, int Bo) {
+void do_interp_output(batotp_ctx *h, const BatchRun &r, int b0, int Bo) {
   const DevCfg &c = h->cfg;
-  ensure_out(h, Bo);
+  ensure_out(h, r, Bo);
   Ws &w = h->w;
   w.b0 = b0;
   w.Bo = Bo;
@@ -1362,33 +1375,34 @@ void do_interp_output(batotp_ctx *h, int b0, int Bo) {
     if (c.trqOn) thomas_rows(h, trqCur, w.TrqM, Bo, b0, c.J, MAXD, 2, 0);
   }
   const bool strictQuat = (c.C == 7 && c.c.trig_mode != 0);
-  const int rp = row_pitch(h), hp = hist_pitch(h);
+  const int rp = row_pitch(h, r), hp = hist_pitch(h, r);
+  OutSet &o = *h->outSet;
   const long long *rag = nullptr;
   long long rag0 = 0;
-  if (h->ragged) {
+  if (r.ragged) {
     // ragged layout: the chunk's block offsets were computed on the host from the sweep results (plan_ragged: the
     // output length is a function of the step count) and uploaded once; the sub-chunk's blocks are packed back to
     // back in the staging set, i.e. relative to the first of them
     rag = h->w.ragOff + b0;
     rag0 = h->ragOffHost[b0];
-    h->ragBase[h->curSet] = h->ragChunkBase + rag0;
-    h->ragTotal[h->curSet] = h->ragOffHost[b0 + Bo] - rag0;
+    o.ragBase = h->ragChunkBase + rag0;
+    o.ragTotal = h->ragOffHost[b0 + Bo] - rag0;
   }
-  float *cartDst = h->ragged ? (float *)nullptr : h->d_cartOut;
+  float *cartDst = r.ragged ? (float *)nullptr : o.cart;
   if (c.c.robot_type == BATOTP_GENJNT && c.C != 7 && c.Cin <= MAXD && !c.trqOn && !h->d_outD && rp > 0 && Bo > 0) {
     // generic robot, float rows only: warp-per-tile staging through shared memory (k_out_pack_rows)
     const long long rows = cdiv(Bo, OP_WARPS);
     const long long gy = std::min<long long>(rows, 32768), gz = (rows + gy - 1) / gy;
     ProfScope ps_(h, "k_out_pack_rows");
     BATOTP_LAUNCH_WARP(k_out_pack_rows, dim3((unsigned)cdiv(rp, 32), (unsigned)gy, (unsigned)gz),
-                       dim3(32, OP_WARPS, 1), 0, h->stream, w, cur, w.OM, h->d_thetaOut, cartDst, rp, rag, rag0, rp, Bo);
+                       dim3(32, OP_WARPS, 1), 0, h->stream, w, cur, w.OM, o.theta, cartDst, rp, rag, rag0, rp, Bo);
     g_check_launch();
     h->launches++;
   } else {
-    LAUNCH_PT(h, k_out_pack, std::max(w.OutC, rp), Bo, w, cur, w.OM, trqCur, w.TrqM, h->d_thetaOut, cartDst,
-              h->d_trqOut, strictQuat ? h->d_cartOutD : (double *)nullptr, h->d_outD, rp, rag, rag0);
+    LAUNCH_PT(h, k_out_pack, std::max(w.OutC, rp), Bo, w, cur, w.OM, trqCur, w.TrqM, o.theta, cartDst, o.trq,
+              strictQuat ? h->d_cartOutD : (double *)nullptr, h->d_outD, rp, rag, rag0);
   }
-  LAUNCH_PT(h, k_pack_hist, std::max(w.Sc, hp), Bo, w, h->d_histOut, hp);
+  LAUNCH_PT(h, k_pack_hist, std::max(w.Sc, hp), Bo, w, o.hist, hp);
   h->phase = 4;
 }
 
@@ -1604,9 +1618,9 @@ int batotp_cuda_create(int device, batotp_handle *out) {
     delete h;
     return -1;
   }
-  for (int q = 0; q < NSETS; ++q)
-    if (cudaEventCreateWithFlags(&h->evOut[q], cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->evCopied[q], cudaEventDisableTiming) != cudaSuccess) {
+  for (OutSet &o : h->sets)
+    if (cudaEventCreateWithFlags(&o.packed, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&o.copied, cudaEventDisableTiming) != cudaSuccess) {
       delete h;
       return -1;
     }
@@ -1632,9 +1646,9 @@ int batotp_cuda_destroy(batotp_handle h) {
 #ifndef BATOTP_HOST_EMU
   cudaStreamDestroy(h->stream);
   cudaStreamDestroy(h->copyStream);
-  for (int q = 0; q < NSETS; ++q) {
-    if (h->evOut[q]) cudaEventDestroy(h->evOut[q]);
-    if (h->evCopied[q]) cudaEventDestroy(h->evCopied[q]);
+  for (OutSet &o : h->sets) {
+    if (o.packed) cudaEventDestroy(o.packed);
+    if (o.copied) cudaEventDestroy(o.copied);
   }
 #endif
   delete h;
@@ -1645,7 +1659,7 @@ const char *batotp_cuda_last_error(batotp_handle h) { return h ? h->err.c_str() 
 
 int batotp_cuda_set_chunk(batotp_handle h, int chunk) {
   if (!h || chunk < 0) return -1;
-  h->chunk = chunk;
+  h->opt.chunk = chunk;
   h->learnedChunk = 0;
   return 0;
 }
@@ -1777,7 +1791,7 @@ int batotp_cuda_selftest_trig(batotp_handle h, unsigned long long seed, long lon
 
 int batotp_cuda_set_keep_f64(batotp_handle h, int on) {
   if (!h) return -1;
-  h->keepF64 = on != 0;
+  h->opt.keepF64 = on != 0;
   return 0;
 }
 
@@ -1809,7 +1823,7 @@ int batotp_cuda_stats_reset(batotp_handle h) {
 }
 int batotp_cuda_set_profile(batotp_handle h, int on) {
   if (!h) return -1;
-  h->profile = on != 0;
+  h->opt.profile = on != 0;
   h->prof.clear();
   return 0;
 }
@@ -1843,7 +1857,10 @@ int batotp_emu_set_rcp_ulps(int k) {
 // arrays were allocated for: {chunk, out, perTraj, wsBytes, outBytes, B}
 int batotp_emu_workspace_plan(batotp_handle h, size_t *out) {
   if (!h || !out) return -1;
-  const Footprints fp = footprints(h, h->wsHeld);
+  BatchRun r;  // at the pitches the held output arrays were allocated for
+  r.rowPitch = h->outHeld.rowP;
+  r.histPitch = h->outHeld.histP;
+  const Footprints fp = footprints(h, r, h->wsHeld);
   const size_t v[6] = {fp.chunk, fp.out, fp.perTraj, h->wsBytes, h->outBytes, (size_t)h->wsHeld.B};
   memcpy(out, v, sizeof v);
   return 0;
@@ -1957,14 +1974,14 @@ static int load_chunk(batotp_handle h, const batotp_cfg *cfg, const batotp_batch
 }
 
 // one chunk through interpInputData with capacity planning / retry
-static int chunk_interp_input(batotp_handle h, bool haveN0) {
+static int chunk_interp_input(batotp_handle h, const BatchRun &r, bool haveN0) {
   int Nc = std::max(h->hwNc, h->n0max + 8);
   bool plan = (h->hwNc == 0);
   for (int attempt = 0; attempt < 8; ++attempt) {
     // the step capacity follows the grid the planning pass finds (a sweep takes about as many steps as the
     // grid has points; twice that leaves room), or what earlier chunks needed
-    const int Sc = std::min(h->maxSteps, std::max(h->hwSc, h->stepHint > 0 ? h->stepHint : std::max(1024, 2 * Nc)));
-    ensure_ws(h, h->B, Nc, Sc);
+    const int Sc = std::min(h->opt.maxSteps, std::max(h->hwSc, h->opt.stepHint > 0 ? h->opt.stepHint : std::max(1024, 2 * Nc)));
+    ensure_ws(h, r, h->B, Nc, Sc);
     h->w.B = h->B;
     const int need = do_interp_input(h, haveN0, plan);
     if (need > 0) {  // planning pass asked for more room
@@ -1987,11 +2004,11 @@ static int chunk_interp_input(batotp_handle h, bool haveN0) {
 }
 
 // Ragged result layout: the output length of a trajectory follows from its forward sweep (ba.cpp:1664-1685 output
-// resolution, 1838-1871 smoothing / decimation, 1873-1921 final sizes - the arithmetic of k_out_plan,
-// k_out_smooth_plan and k_out_final_plan), so the host lays the chunk's blocks out as soon as the sweeps are back:
-// prefix sums -> w.ragOff, and the chunk's place in the caller's buffers from the shared counter.  (A trajectory
-// the output phase rejects later keeps its reserved block and reports n_out = 0.)
-static void plan_ragged(batotp_handle h) {
+// resolution, then out_n_over, out_n_sm and out_n_final as in k_out_plan, k_out_smooth_plan and k_out_final_plan),
+// so the host lays the chunk's blocks out as soon as the sweeps are back: prefix sums -> w.ragOff, and the chunk's
+// place in the caller's buffers from the shared counter.  (A trajectory the output phase rejects later keeps its
+// reserved block and reports n_out = 0.)
+static void plan_ragged(batotp_handle h, const BatchRun &r) {
   const batotp_cfg &c = h->cfg.c;
   const int B = h->B;
   h->ragOffHost.resize((size_t)B + 1);
@@ -2009,18 +2026,16 @@ static void plan_ragged(batotp_handle h) {
       outSmooth *= std::max(outResT / outRes, 1.);
     }
     const double tLast = s.tStep * (double)(s.nFwd - 1);
-    int nOver = (int)(outSmooth * std::ceil(tLast / outRes + 1.));
-    nOver = std::max(nOver, 4);
-    const int nSm = outSmooth > 1.5 ? std::max((int)((nOver - 1) / outSmooth) + 1, 4) : nOver;
-    const int nOut = re ? std::max((int)(std::ceil(tLast / outResT)), 4) : nSm;
-    acc += nOut;
+    const int nSm = out_n_sm(out_n_over(tLast, outRes, outSmooth), outSmooth);
+    acc += out_n_final(tLast, outResT, re, nSm);
   }
   h->ragOffHost[B] = acc;
-  h->ragChunkBase = h->ragNext->fetch_add(acc);
+  h->ragChunkBase = r.ragNext->fetch_add(acc);
   g_h2d(h->w.ragOff, h->ragOffHost.data(), ((size_t)B + 1) * sizeof(long long), h->stream);
 }
 
-static int chunk_sweeps_output(batotp_handle h, bool haveN0) {
+// (`at`: the chunk's first trajectory in the caller's batch, which names its stragglers)
+static int chunk_sweeps_output(batotp_handle h, BatchRun &r, int at, bool haveN0) {
   for (int attempt = 0; attempt < 10; ++attempt) {
     if (do_sweeps(h) != 0) return -1;
     h->hst.resize(h->B);
@@ -2045,32 +2060,22 @@ static int chunk_sweeps_output(batotp_handle h, bool haveN0) {
       mxF = std::max(mxF, std::max(h->hst[b].nFwd, h->hst[b].nRev));
     }
     h->mxSteps = mxF;
-    if (stepCap && h->collectStragglers && nCap <= std::max(8, h->B / 64) && h->w.Sc < h->maxSteps) {
+    if (stepCap && r.collect && nCap <= std::max(8, h->B / 64) && h->w.Sc < h->opt.maxSteps) {
       // a few trajectories outgrew a capacity that serves the rest of the chunk: they keep BATOTP_ST_STEP_CAP for
       // now (the output phase skips them) and are re-run together after the chunks of the batch, instead of the
       // whole chunk being redone with twice the capacity for their sake
       for (int b = 0; b < h->B; ++b)
         if ((h->hst[b].status & ST_STEP_CAP) && !(h->hst[b].status & (ST_FATAL_MASK & ~ST_STEP_CAP)))
-          h->stragglers.push_back(h->chunkFirst + b);
-      h->stragglerSc = std::max(h->stragglerSc, h->w.Sc);
+          r.stragglers.push_back(at + b);
+      r.stragglerSc = std::max(r.stragglerSc, h->w.Sc);
       stepCap = false;
-    }
-    if (!stepCap) {
-      for (int b = 0; b < h->B; ++b) {
-        const TrajState &t = h->hst[b];
-        if (t.status & ST_FATAL_MASK) continue;
-        h->cntVerify += t.nVerify;
-        h->cntSteps += (t.nRev - 1) + (t.nFwd - 1);
-        h->cntTraj++;
-      }
-      h->hwSc = std::max(h->hwSc, std::min(h->w.Sc, (int)(mxF * 1.25) + 64));
-      if (h->ragged) plan_ragged(h);
-      return 0;
     }
     // A trajectory that crawls (e.g. an infeasible path whose bisection keeps failing, ba.cpp:1307-1319) runs
     // until maxIntegTime in the reference.  The step capacity follows it up to maxSteps; beyond that the
-    // trajectory keeps BATOTP_ST_STEP_CAP (reported as not optimised) instead of holding the batch hostage.
-    if ((long long)h->w.Sc * 2 > (long long)h->maxSteps) {
+    // trajectory keeps BATOTP_ST_STEP_CAP (reported as not optimised) instead of holding the batch hostage: the
+    // chunk is accepted, and the next chunks start with this capacity (one pass each).
+    const bool atCeiling = stepCap && (long long)h->w.Sc * 2 > (long long)h->opt.maxSteps;
+    if (!stepCap || atCeiling) {
       for (int b = 0; b < h->B; ++b) {
         const TrajState &t = h->hst[b];
         if (t.status & ST_FATAL_MASK) continue;
@@ -2078,14 +2083,14 @@ static int chunk_sweeps_output(batotp_handle h, bool haveN0) {
         h->cntSteps += (t.nRev - 1) + (t.nFwd - 1);
         h->cntTraj++;
       }
-      h->hwSc = std::max(h->hwSc, h->w.Sc);  // the next chunks start with this capacity: one pass each
-      if (h->ragged) plan_ragged(h);
+      h->hwSc = std::max(h->hwSc, atCeiling ? h->w.Sc : std::min(h->w.Sc, (int)(mxF * 1.25) + 64));
+      if (r.ragged) plan_ragged(h, r);
       return 0;
     }
     // grow the step capacity and redo the chunk from the start (the status word is sticky)
     const int Sc = h->w.Sc * 2;
     const int Nc = h->w.Nc;
-    ensure_ws(h, h->B, Nc, Sc);
+    ensure_ws(h, r, h->B, Nc, Sc);
     h->w.B = h->B;
     const int need = do_interp_input(h, haveN0, false);
     (void)need;
@@ -2099,10 +2104,6 @@ int batotp_cuda_load(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_
   try {
     h->lastHaveN0 = in->n0 != nullptr;
     h->inSet[0].src = h->inSet[1].src = nullptr;
-    h->rowPitch = h->histPitch = 0;  // phase-wise calls pack at the device capacities
-    h->ragged = false;
-    h->chunkFirst = 0;
-    h->collectStragglers = false;
     const int rc = load_chunk(h, cfg, in, 0, in->B);
     if (rc == 0) g_sync(h->stream);  // the caller's arrays are free again when this call returns
     return rc;
@@ -2114,8 +2115,9 @@ int batotp_cuda_load(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_
 int batotp_cuda_interp_input(batotp_handle h) {
   if (!h || h->phase < 1) return -1;
   try {
-    if (h->cfg.c.is_interp_only) return do_interp_only(h, h->lastHaveN0);  // result ready for batotp_cuda_fetch
-    return chunk_interp_input(h, h->lastHaveN0);
+    const BatchRun r;
+    if (h->cfg.c.is_interp_only) return do_interp_only(h, r, h->lastHaveN0);  // result ready for batotp_cuda_fetch
+    return chunk_interp_input(h, r, h->lastHaveN0);
   } catch (const Err &e) {
     h->err = e.msg;
     return -1;
@@ -2124,7 +2126,8 @@ int batotp_cuda_interp_input(batotp_handle h) {
 int batotp_cuda_sweeps(batotp_handle h) {
   if (!h || h->phase < 2) return -1;
   try {
-    return chunk_sweeps_output(h, h->lastHaveN0);
+    BatchRun r;
+    return chunk_sweeps_output(h, r, 0, h->lastHaveN0);
   } catch (const Err &e) {
     h->err = e.msg;
     return -1;
@@ -2133,8 +2136,8 @@ int batotp_cuda_sweeps(batotp_handle h) {
 int batotp_cuda_interp_output(batotp_handle h) {
   if (!h || h->phase < 3) return -1;
   try {
-    if (h->B > h->outChunk) h->outChunk = h->B;  // the phase-wise API keeps one sub-chunk resident
-    do_interp_output(h, 0, h->B);
+    if (h->B > h->opt.outChunk) h->opt.outChunk = h->B;  // the phase-wise API keeps one sub-chunk resident
+    do_interp_output(h, BatchRun(), 0, h->B);
     g_sync(h->stream);
     return 0;
   } catch (const Err &e) {
@@ -2181,17 +2184,19 @@ static void copy_rows(void *dst, size_t want, const void *src, size_t dp, size_t
     g_d2h_2d(dst, want * es, src, dp * es, std::min(want, dp) * es, rows, cs);
 }
 
-// packed float32 rows / histories / flags of the current output sub-chunk -> the caller's buffers (host or
+// packed float32 rows / histories / flags of the current output sub-chunk -> the caller's buffers r.out (host or
 // device memory), enqueued on stream `cs` (the staging set is the one selected when the sub-chunk was packed)
-static void fetch_rows(batotp_handle h, batotp_batch_out *out, int first, cudaStream_t cs) {
+static void fetch_rows(batotp_handle h, const BatchRun &r, int first, cudaStream_t cs) {
   const DevCfg &c = h->cfg;
   const Ws &w = h->w;
+  const OutSet &o = *h->outSet;
+  batotp_batch_out *out = r.out;
   const int Bo = w.Bo, g0 = first + w.b0;
-  const size_t oc = (size_t)out->out_cap, rp = (size_t)row_pitch(h);
-  if (h->ragged) {
+  const size_t oc = (size_t)out->out_cap, rp = (size_t)row_pitch(h, r);
+  if (r.ragged) {
     // the sub-chunk's blocks, back to back in the staging set -> their place in the caller's buffer, in one copy;
     // the offsets were computed when the sub-chunk was packed (do_interp_output)
-    const long long base = h->ragBase[h->curSet], total = h->ragTotal[h->curSet];
+    const long long base = o.ragBase, total = o.ragTotal;
     if (base + total > out->ragged_cap) {
       char buf[160];
       snprintf(buf, sizeof buf, "ragged_cap (%lld points) is too small: %lld points needed so far", out->ragged_cap,
@@ -2200,34 +2205,35 @@ static void fetch_rows(batotp_handle h, batotp_batch_out *out, int first, cudaSt
     }
     for (int bl = 0; bl < Bo; ++bl) out->row_offset[g0 + bl] = h->ragChunkBase + h->ragOffHost[w.b0 + bl];
     if (out->theta_out && total > 0)
-      g_d2h(out->theta_out + (size_t)base * c.J, h->d_thetaOut, (size_t)total * c.J * 4, cs);
+      g_d2h(out->theta_out + (size_t)base * c.J, o.theta, (size_t)total * c.J * 4, cs);
     if (out->trq_out && c.trqOn && total > 0)
-      g_d2h(out->trq_out + (size_t)base * c.J, h->d_trqOut, (size_t)total * c.J * 4, cs);
+      g_d2h(out->trq_out + (size_t)base * c.J, o.trq, (size_t)total * c.J * 4, cs);
   } else {
     if (out->theta_out && oc > 0)
-      copy_rows(out->theta_out + (size_t)g0 * c.J * oc, oc, h->d_thetaOut, rp, (size_t)Bo * c.J, 4, cs);
+      copy_rows(out->theta_out + (size_t)g0 * c.J * oc, oc, o.theta, rp, (size_t)Bo * c.J, 4, cs);
     if (out->trq_out && oc > 0 && c.trqOn)
-      copy_rows(out->trq_out + (size_t)g0 * c.J * oc, oc, h->d_trqOut, rp, (size_t)Bo * c.J, 4, cs);
+      copy_rows(out->trq_out + (size_t)g0 * c.J * oc, oc, o.trq, rp, (size_t)Bo * c.J, 4, cs);
   }
   if (out->cart_out && oc > 0 && c.Cin > 0 && !(c.C == 7 && c.c.trig_mode != 0))
-    copy_rows(out->cart_out + (size_t)g0 * c.Cin * oc, oc, h->d_cartOut, rp, (size_t)Bo * c.Cin, 4, cs);
-  const size_t hc = (size_t)out->hist_cap, hp = (size_t)hist_pitch(h);
-  if (out->hist && hc > 0) copy_rows(out->hist + (size_t)g0 * 4 * hc, hc, h->d_histOut, hp, (size_t)Bo * 4, 4, cs);
+    copy_rows(out->cart_out + (size_t)g0 * c.Cin * oc, oc, o.cart, rp, (size_t)Bo * c.Cin, 4, cs);
+  const size_t hc = (size_t)out->hist_cap, hp = (size_t)hist_pitch(h, r);
+  if (out->hist && hc > 0) copy_rows(out->hist + (size_t)g0 * 4 * hc, hc, o.hist, hp, (size_t)Bo * 4, 4, cs);
   if (out->flags && hc > 0)
     copy_rows(out->flags + (size_t)g0 * 2 * hc, hc, w.flags + (size_t)w.b0 * 2 * w.Sc, (size_t)w.Sc, (size_t)Bo * 2, 1, cs);
 }
 
-// copy the results of the current output sub-chunk [w.b0, w.b0+w.Bo) to the caller's buffers;
+// copy the results of the current output sub-chunk [w.b0, w.b0+w.Bo) to the caller's buffers r.out;
 // `first` = index of the resident chunk's first trajectory in the caller's batch
-static void fetch_sub(batotp_handle h, batotp_batch_out *out, int first) {
+static void fetch_sub(batotp_handle h, const BatchRun &r, int first) {
   const DevCfg &c = h->cfg;
   const Ws &w = h->w;
+  batotp_batch_out *out = r.out;
   ProfScope ps_(h, "copy_d2h(fetch)");
   const bool strictQuatOut = out->cart_out && out->out_cap > 0 && c.Cin > 0 && c.C == 7 && c.c.trig_mode != 0;
   if (out->on_device && strictQuatOut)
     throw Err{"batotp_batch_out.on_device: axis-angle rows in strict-trig mode are finished on the host; use trig_mode 0"};
   fetch_scalars(h, out, first, w.b0, w.Bo);
-  fetch_rows(h, out, first, h->stream);
+  fetch_rows(h, r, first, h->stream);
   if (strictQuatOut) host_q2aa_out(h, out, first + w.b0);
   g_sync(h->stream);
 }
@@ -2235,7 +2241,9 @@ static void fetch_sub(batotp_handle h, batotp_batch_out *out, int first) {
 int batotp_cuda_fetch(batotp_handle h, batotp_batch_out *out) {
   if (!h || !out || h->phase < 4) return -1;
   try {
-    fetch_sub(h, out, 0);
+    BatchRun r;
+    r.out = out;
+    fetch_sub(h, r, 0);
     return 0;
   } catch (const Err &e) {
     h->err = e.msg;
@@ -2243,17 +2251,14 @@ int batotp_cuda_fetch(batotp_handle h, batotp_batch_out *out) {
   }
 }
 
-// one resident chunk [at, at+B) of the caller's batch through the whole path
-static void process_chunk(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_in *in, batotp_batch_out *out,
-                          int at, int B, int nextB) {
-  if (load_chunk(h, cfg, in, at, B) != 0) throw Err{h->err};
+// one resident chunk [at, at+B) of the caller's batch through the whole path (loadCfg: set the run's configuration
+// first)
+static void process_chunk(batotp_handle h, BatchRun &r, bool loadCfg, int at, int B, int nextB) {
+  const batotp_batch_in *in = r.in;
+  batotp_batch_out *out = r.out;
+  if (load_chunk(h, loadCfg ? r.cfg : nullptr, in, at, B) != 0) throw Err{h->err};
   h->lastHaveN0 = in->n0 != nullptr;
-  h->chunkFirst = at;
-  // the staging sets are packed at the caller's pitches: a sub-chunk then leaves in one contiguous copy
-  h->ragged = out->row_offset != nullptr && h->ragNext != nullptr;
-  h->rowPitch = (!h->ragged && (out->theta_out || out->cart_out || out->trq_out) && out->out_cap > 0) ? out->out_cap : 0;
-  h->histPitch = (out->hist && out->hist_cap > 0) ? out->hist_cap : 0;
-  if (nextB > 0 && !in->on_device && !h->profile) {
+  if (nextB > 0 && !in->on_device && !h->opt.profile) {
     // the host rows of the next chunk travel while this one is computed
     try {
       issue_inputs(h, in, at + B, nextB, h->curIn ^ 1, h->copyStream, true);
@@ -2262,48 +2267,48 @@ static void process_chunk(batotp_handle h, const batotp_cfg *cfg, const batotp_b
     }
   }
   if (h->cfg.c.is_interp_only) {  // ba.cpp:139-159: re-sample only
-    if (do_interp_only(h, h->lastHaveN0) != 0) throw Err{h->err};
-    fetch_sub(h, out, at);
+    if (do_interp_only(h, r, h->lastHaveN0) != 0) throw Err{h->err};
+    fetch_sub(h, r, at);
     return;
   }
-  if (chunk_interp_input(h, h->lastHaveN0) != 0) throw Err{h->err};
-  if (h->beforeSweeps) h->beforeSweeps();
+  if (chunk_interp_input(h, r, h->lastHaveN0) != 0) throw Err{h->err};
+  if (r.beforeSweeps) r.beforeSweeps();
   if (h->copiesPending && out->flags && out->hist_cap > 0) {
     // the switching flags travel straight out of the chunk workspace, which the sweeps overwrite: when they were
     // asked for, the sweeps queue up behind the previous chunk's copies.  (Rows and histories leave from the
     // staging sets, which only the output phase touches: their copies go on beside the next chunk's sweeps.)
-    for (int q = 0; q < NSETS; ++q)
-      if (h->setBusy[q]) {
-        g_stream_wait(h->stream, h->evCopied[q]);
-        h->setBusy[q] = false;
+    for (OutSet &o : h->sets)
+      if (o.busy) {
+        g_stream_wait(h->stream, o.copied);
+        o.busy = false;
       }
     h->copiesPending = false;
   }
-  if (chunk_sweeps_output(h, h->lastHaveN0) != 0) throw Err{h->err};
-  if (h->onSweepsDone) h->onSweepsDone();
+  if (chunk_sweeps_output(h, r, at, h->lastHaveN0) != 0) throw Err{h->err};
+  if (r.onSweepsDone) r.onSweepsDone();
   {
       const DevCfg &c = h->cfg;
       const bool strictQuatOut = out->cart_out && out->out_cap > 0 && c.Cin > 0 && c.C == 7 && c.c.trig_mode != 0;
-      if (strictQuatOut || h->profile) {  // host post-processing per sub-chunk / serialised measurement
-        for (int b0 = 0; b0 < B; b0 += h->outChunk) {
-          do_interp_output(h, b0, std::min(h->outChunk, B - b0));
-          fetch_sub(h, out, at);
+      if (strictQuatOut || h->opt.profile) {  // host post-processing per sub-chunk / serialised measurement
+        for (int b0 = 0; b0 < B; b0 += h->opt.outChunk) {
+          do_interp_output(h, r, b0, std::min(h->opt.outChunk, B - b0));
+          fetch_sub(h, r, at);
         }
       } else {
         // rows of sub-chunk k go to the host on the copy stream while sub-chunk k+1 is computed into the
         // other staging set
-        for (int b0 = 0; b0 < B; b0 += h->outChunk) {
-          ensure_out(h, std::min(h->outChunk, B - b0));
-          const int q = h->setNext;
-          h->setNext = (q + 1) % NSETS;
-          if (h->setBusy[q]) g_stream_wait(h->stream, h->evCopied[q]);  // the set's last rows have reached the host
-          select_out_set(h, q);
-          do_interp_output(h, b0, std::min(h->outChunk, B - b0));
-          g_event_record(h->evOut[q], h->stream);
-          g_stream_wait(h->copyStream, h->evOut[q]);
-          fetch_rows(h, out, at, h->copyStream);
-          g_event_record(h->evCopied[q], h->copyStream);
-          h->setBusy[q] = true;
+        for (int b0 = 0; b0 < B; b0 += h->opt.outChunk) {
+          ensure_out(h, r, std::min(h->opt.outChunk, B - b0));
+          OutSet &o = h->sets[h->setNext];
+          h->setNext = (h->setNext + 1) % NSETS;
+          if (o.busy) g_stream_wait(h->stream, o.copied);  // the set's last rows have reached the host
+          h->outSet = &o;
+          do_interp_output(h, r, b0, std::min(h->opt.outChunk, B - b0));
+          g_event_record(o.packed, h->stream);
+          g_stream_wait(h->copyStream, o.packed);
+          fetch_rows(h, r, at, h->copyStream);
+          g_event_record(o.copied, h->copyStream);
+          o.busy = true;
         }
         fetch_scalars(h, out, at, 0, B);
         h->copiesPending = true;  // waited for before the next chunk's sweeps, or before the call returns
@@ -2313,7 +2318,7 @@ static void process_chunk(batotp_handle h, const batotp_cfg *cfg, const batotp_b
 
 int batotp_cuda_set_tail_overlap(batotp_handle h, int on) {
   if (!h) return -1;
-  h->tailOverlap = on != 0;
+  h->opt.tailOverlap = on != 0;
   return 0;
 }
 
@@ -2329,12 +2334,12 @@ static void sync_quiet(batotp_handle h) {
 // trajectories per round of the sweep kernel a chunk of B trajectories of this configuration would take (0: not known)
 static int sweep_round_capacity(batotp_handle h, const batotp_cfg *cfg, int B) {
   if (!h->haveCfg || memcmp(&h->cfg.c, cfg, sizeof(batotp_cfg)) != 0) return 0;  // learnt for another configuration
-  return h->sweepCap[group_sweep(h->cfg, h->sweepKernel, B) ? 1 : 0];
+  return h->sweepCap[group_sweep(h->cfg, h->opt.sweepKernel, B) ? 1 : 0];
 }
 
-// The chunks [0, mainB) of a batch on context h, one after the other (out-of-memory: smaller chunks)
-static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_in *in, batotp_batch_out *out,
-                       int from, int mainB, int &chunk, bool &first) {
+// The chunks [from, mainB) of a batch on context h, one after the other (out-of-memory: smaller chunks)
+static void run_chunks(batotp_handle h, BatchRun &r, int from, int mainB, int &chunk, bool &first) {
+  const batotp_cfg *cfg = r.cfg;
   for (int at = from; at < mainB;) {
     // A sweep launch lasts whole rounds of the trajectories it keeps resident (it is bound by the latency of one
     // trajectory), so a chunk of 1.5 rounds pays for 2 (CSPR3DOF on the B200: 9472 paths per round; memory allows
@@ -2342,7 +2347,7 @@ static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batc
     // last one of its batch is cut to whole rounds - what it leaves moves on to the next chunk - and the last one when
     // its final round would be less than a quarter full (a fuller round is cheaper than another chunk).
     auto whole_rounds = [&](int n, int left) {
-      const int cap = h->chunk == 0 ? sweep_round_capacity(h, cfg, n) : 0;  // (an explicit chunk setting is taken literally)
+      const int cap = h->opt.chunk == 0 ? sweep_round_capacity(h, cfg, n) : 0;  // (an explicit chunk setting is taken literally)
       if (cap <= 0 || n <= cap) return n;
       return (left > n || n % cap < cap / 4) ? n / cap * cap : n;
     };
@@ -2353,7 +2358,7 @@ static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batc
       fprintf(stderr, "[batotp] chunk at %d: %d paths (chunk setting %d, round capacity %d; capB %d capNc %d capSc %d; alloc %.1f ms free %.1f ms so far)\n",
               at, B, chunk, sweep_round_capacity(h, cfg, B), h->wsHeld.B, h->wsHeld.Nc, h->wsHeld.Sc, g_allocMs, g_freeMs);
     try {
-      process_chunk(h, first ? cfg : nullptr, in, out, at, B, nextB);
+      process_chunk(h, r, first, at, B, nextB);
     } catch (const Err &e) {
       // a workspace did not fit (long paths, many rows): release everything and go on with smaller chunks
       if (!e.oom) throw;
@@ -2366,17 +2371,17 @@ static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batc
         free_ws(h);
         free_out(h);
       }
-      const int chunk0 = chunk, out0 = h->outChunk;
+      const int chunk0 = chunk, out0 = h->opt.outChunk;
       if (e.fitB > 0 && e.fitB < B)  // the workspace planner knows what fits
         chunk = std::max(1, e.fitB >= SW_NT ? e.fitB / SW_NT * SW_NT : e.fitB);
-      else if (h->allocPhase == 1 && std::min(h->outChunk, B) > 1)
-        h->outChunk = std::max(1, std::min(h->outChunk, B) / 2);
+      else if (h->allocPhase == 1 && std::min(h->opt.outChunk, B) > 1)
+        h->opt.outChunk = std::max(1, std::min(h->opt.outChunk, B) / 2);
       else
         chunk = std::max(1, B > 2 * SW_NT ? (B / 2 + SW_NT - 1) / SW_NT * SW_NT : B / 2);
-      if ((chunk >= chunk0 || chunk >= B) && h->outChunk >= std::min(out0, B)) throw;  // nothing left to shrink
+      if ((chunk >= chunk0 || chunk >= B) && h->opt.outChunk >= std::min(out0, B)) throw;  // nothing left to shrink
       continue;
     }
-    if (g_trace()) fprintf(stderr, "[batotp]   done in %.1f ms (Nc %d Sc %d, stragglers so far %zu)\n", g_now_ms() - tC0, h->w.Nc, h->w.Sc, h->stragglers.size());
+    if (g_trace()) fprintf(stderr, "[batotp]   done in %.1f ms (Nc %d Sc %d, stragglers so far %zu)\n", g_now_ms() - tC0, h->w.Nc, h->w.Sc, r.stragglers.size());
     first = false;
     at += B;
   }
@@ -2386,9 +2391,10 @@ static void run_chunks(batotp_handle h, const batotp_cfg *cfg, const batotp_batc
 // into one small batch and run again with four times that capacity (growing further, up to maxSteps, by the
 // ordinary capacity retries of a chunk); their results replace the BATOTP_ST_STEP_CAP placeholders in the caller's
 // arrays.  Trajectories are independent, so the results are the ones a single large-capacity pass would give.
-static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_in *in, batotp_batch_out *out) {
-  std::vector<int> idx = h->stragglers;
-  h->stragglers.clear();
+static void run_stragglers(batotp_handle h, BatchRun &r) {
+  const batotp_batch_in *in = r.in;
+  batotp_batch_out *out = r.out;
+  std::vector<int> idx = std::move(r.stragglers);
   std::sort(idx.begin(), idx.end());
   idx.erase(std::unique(idx.begin(), idx.end()), idx.end());
   const int n = (int)idx.size();
@@ -2453,7 +2459,7 @@ static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_
   // (ragged layout: the stragglers are computed into a pitched temporary wide enough for the step ceiling and
   // appended to the caller's buffer block by block)
   const bool ragOut = out->row_offset != nullptr;
-  const size_t oc = ragOut ? (size_t)final_cap(h, h->maxSteps, 0) : (size_t)out->out_cap, hc = (size_t)out->hist_cap;
+  const size_t oc = ragOut ? (size_t)final_cap(h, h->opt.maxSteps, 0) : (size_t)out->out_cap, hc = (size_t)out->hist_cap;
   std::vector<int> oI[6];
   std::vector<double> oD[4];
   for (auto &v : oI) v.assign(n, 0);
@@ -2479,14 +2485,11 @@ static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_
   if (out->trq_out && oc && c.trqOn) { oTq.assign((size_t)n * J * oc, 0.f); o2.trq_out = oTq.data(); }
   if (out->hist && hc) { oHist.assign((size_t)n * 4 * hc, 0.f); o2.hist = oHist.data(); }
   if (out->flags && hc) { oFl.assign((size_t)n * 2 * hc, 0); o2.flags = oFl.data(); }
-  // ---- run them as one chunk with a larger step capacity; the capacity marks of the batch are put back after
-  std::atomic<long long> *const keepRag = h->ragNext;
-  h->ragNext = nullptr;  // the temporary is pitched
+  // ---- run them as one chunk with a larger step capacity (a run of their own: pitched, collecting nothing); the
+  // capacity mark of the batch is put back after
+  BatchRun r2(r.cfg, &in2, &o2, nullptr, false);
   const int keepHwSc = h->hwSc;
-  const bool keepCollect = h->collectStragglers;
-  h->collectStragglers = false;
-  h->hwSc = (int)std::min<long long>(h->maxSteps, (long long)std::max(h->stragglerSc, 1024) * 4);
-  h->stragglerSc = 0;
+  h->hwSc = (int)std::min<long long>(h->opt.maxSteps, (long long)std::max(r.stragglerSc, 1024) * 4);
   g_sync(h->stream);
   g_sync(h->copyStream);
   h->copiesPending = false;
@@ -2494,19 +2497,15 @@ static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_
   try {
     int chunk2 = n;
     bool first2 = true;
-    run_chunks(h, cfg, &in2, &o2, 0, n, chunk2, first2);  // (with its out-of-memory retries)
+    run_chunks(h, r2, 0, n, chunk2, first2);  // (with its out-of-memory retries)
     g_sync(h->copyStream);
     g_sync(h->stream);
     h->copiesPending = false;
   } catch (...) {
     h->hwSc = keepHwSc;
-    h->collectStragglers = keepCollect;
-    h->ragNext = keepRag;
     throw;
   }
   h->hwSc = keepHwSc;
-  h->collectStragglers = keepCollect;
-  h->ragNext = keepRag;
   free_ws(h);  // the large-capacity workspace is not what the next batch needs
   free_out(h);
   // ---- scatter
@@ -2527,7 +2526,7 @@ static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_
       if (dD[q]) put(dD[q] + g, &oD[q][k], sizeof(double));
     if (ragOut) {
       const long long nn = oI[3][k];  // n_out
-      const long long base = keepRag->fetch_add(nn);
+      const long long base = r.ragNext->fetch_add(nn);
       if (base + nn > out->ragged_cap) throw Err{"ragged_cap is too small for the re-run stragglers"};
       out->row_offset[g] = base;
       for (int r = 0; r < J; ++r) {
@@ -2554,39 +2553,27 @@ static void run_stragglers(batotp_handle h, const batotp_cfg *cfg, const batotp_
 int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_in *in,
                                batotp_batch_out *out) {
   if (!h || !cfg || !in || !out) return -1;
-  std::atomic<long long> ragCounter{0};  // ragged layout: the next free point of the caller's row buffers
-  h->ragNext = nullptr;
-  if (out->row_offset) {
-    if (out->on_device || out->cart_out || !out->theta_out || out->ragged_cap <= 0 || cfg->is_interp_only) {
-      h->err = "ragged rows (row_offset): host buffers, theta_out (+ trq_out) only, cart_out = NULL, ragged_cap > 0, "
-               "not with isInterpOnly";
-      return -1;
-    }
-    h->ragNext = &ragCounter;
+  if (out->row_offset &&
+      (out->on_device || out->cart_out || !out->theta_out || out->ragged_cap <= 0 || cfg->is_interp_only)) {
+    h->err = "ragged rows (row_offset): host buffers, theta_out (+ trq_out) only, cart_out = NULL, ragged_cap > 0, "
+             "not with isInterpOnly";
+    return -1;
   }
-  struct RagReset {
-    batotp_ctx *h;
-    ~RagReset() {
-      h->ragNext = nullptr;
-      h->ragged = false;
-      if (h->helper) {
-        h->helper->ragNext = nullptr;
-        h->helper->ragged = false;
-      }
-    }
-  } ragReset{h};
+  std::atomic<long long> ragCounter{0};  // ragged layout: the next free point of the caller's row buffers
+  BatchRun run(cfg, in, out, out->row_offset ? &ragCounter : nullptr, !cfg->is_interp_only);
+  BatchRun tailRun(cfg, in, out, run.ragNext, true);  // the tail chunk's, on the helper context
   bool first = true;
-  int chunk = h->chunk > 0 ? h->chunk : auto_chunk(h, in->B);
+  int chunk = h->opt.chunk > 0 ? h->opt.chunk : auto_chunk(h, in->B);
   const int chunkAuto = chunk;
   // what the workspace planner allowed in the previous call of this configuration: start there (a refused first
   // attempt costs the staging of its inputs)
   const bool sameCfg = h->haveCfg && memcmp(&h->cfg.c, cfg, sizeof(batotp_cfg)) == 0;
-  if (h->chunk == 0 && sameCfg && h->learnedChunk > 0) chunk = std::min(chunk, h->learnedChunk);
+  if (h->opt.chunk == 0 && sameCfg && h->learnedChunk > 0) chunk = std::min(chunk, h->learnedChunk);
   if (!sameCfg) h->learnedChunk = 0;
   {
     // whole rounds of the sweep kernel (run_chunks): applied to the chunk setting itself when the occupancy is already
     // known, so that the tail below is what whole-round chunks leave over
-    const int cap = h->chunk == 0 ? sweep_round_capacity(h, cfg, chunk) : 0;
+    const int cap = h->opt.chunk == 0 ? sweep_round_capacity(h, cfg, chunk) : 0;
     if (cap > 0 && chunk > cap && in->B > chunk) chunk = chunk / cap * cap;
   }
   int mainB = in->B, tail = 0;
@@ -2601,7 +2588,7 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
     cv.notify_all();
   };
   auto finish_tail = [&](int v) {  // every exit path: let the tail thread go (or skip) and wait for it
-    h->onSweepsDone = nullptr;
+    run.onSweepsDone = nullptr;
     if (tailThread.joinable()) {
       signal(v);
       tailThread.join();
@@ -2609,10 +2596,7 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
   };
   try {
     h->inSet[0].src = h->inSet[1].src = nullptr;
-    h->stragglers.clear();
-    h->stragglerSc = 0;
-    h->collectStragglers = !cfg->is_interp_only;
-    if (h->tailOverlap && !h->profile && !out->on_device && !cfg->is_interp_only && in->B > chunk) {
+    if (h->opt.tailOverlap && !h->opt.profile && !out->on_device && !cfg->is_interp_only && in->B > chunk) {
       int sms = 148;
 #ifndef BATOTP_HOST_EMU
       cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
@@ -2624,25 +2608,14 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
           tail = t;
           mainB = in->B - tail;
           batotp_ctx *hp = h->helper;
-          hp->tailOverlap = false;
-          hp->chunk = 0;
-          hp->outChunk = h->outChunk;
-          hp->maxSteps = h->maxSteps;
-          if (hp->stepHint != h->stepHint) hp->hwSc = 0;
-          hp->stepHint = h->stepHint;
-          hp->keepF64 = h->keepF64;
-          hp->sweepKernel = h->sweepKernel;
-          hp->walkerKernel = h->walkerKernel;
-          hp->dynFn = h->dynFn;
-          hp->dynUser = h->dynUser;
-          hp->ragNext = h->ragNext;
-          hp->stragglers.clear();
-          hp->stragglerSc = 0;
-          hp->collectStragglers = true;
-          h->onSweepsDone = [&]() { signal(1); };
+          if (hp->opt.stepHint != h->opt.stepHint) hp->hwSc = 0;
+          hp->opt = h->opt;
+          hp->opt.chunk = 0;
+          hp->opt.tailOverlap = false;
+          run.onSweepsDone = [&]() { signal(1); };
           // the tail's input interpolation runs at once (beside that of the first full chunk); its sweeps wait
           // until the sweeps of the first full chunk have completed, so that they run beside output / input phases
-          hp->beforeSweeps = [&]() {
+          tailRun.beforeSweeps = [&]() {
             std::unique_lock<std::mutex> lk(mu);
             cv.wait(lk, [&] { return go != 0; });
             if (go != 1) throw Err{"tail chunk skipped"};
@@ -2651,18 +2624,15 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
             try {
               hp->inSet[0].src = hp->inSet[1].src = nullptr;
               const bool same = hp->haveCfg && memcmp(&hp->cfg.c, cfg, sizeof(batotp_cfg)) == 0;
-              process_chunk(hp, same ? nullptr : cfg, in, out, mainB, tail, 0);
+              process_chunk(hp, tailRun, !same, mainB, tail, 0);
               g_sync(hp->copyStream);
               hp->copiesPending = false;
-              hp->beforeSweeps = nullptr;
             } catch (const Err &e) {
-              hp->beforeSweeps = nullptr;
               tailRes.failed = true;
               tailRes.oom = e.oom;
               tailRes.msg = e.msg;
               sync_quiet(hp);
             } catch (...) {
-              hp->beforeSweeps = nullptr;
               tailRes.failed = true;
               tailRes.msg = "unexpected exception in the tail chunk";
               sync_quiet(hp);
@@ -2671,8 +2641,8 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
         }
       }
     }
-    run_chunks(h, cfg, in, out, 0, mainB, chunk, first);
-    if (h->chunk == 0 && chunk < chunkAuto) h->learnedChunk = chunk;  // the out-of-memory handling shrank it
+    run_chunks(h, run, 0, mainB, chunk, first);
+    if (h->opt.chunk == 0 && chunk < chunkAuto) h->learnedChunk = chunk;  // the out-of-memory handling shrank it
     finish_tail(1);
     if (tail > 0) {
       batotp_ctx *hp = h->helper;
@@ -2684,25 +2654,22 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
       h->cntTraj += hp->cntTraj;
       h->launches += hp->launches;
       batotp_cuda_stats_reset(hp);
-      h->stragglers.insert(h->stragglers.end(), hp->stragglers.begin(), hp->stragglers.end());
-      h->stragglerSc = std::max(h->stragglerSc, hp->stragglerSc);
-      hp->stragglers.clear();
+      run.stragglers.insert(run.stragglers.end(), tailRun.stragglers.begin(), tailRun.stragglers.end());
+      run.stragglerSc = std::max(run.stragglerSc, tailRun.stragglerSc);
       if (tailRes.failed) {
         if (!tailRes.oom) throw Err{tailRes.msg};
         // no room for the second context's workspaces: release them and run the tail here
         free_ws(hp);
         free_out(hp);
-        run_chunks(h, cfg, in, out, mainB, in->B, chunk, first);
+        run_chunks(h, run, mainB, in->B, chunk, first);
       }
     }
     g_sync(h->copyStream);  // every row has reached the caller's buffers
     h->copiesPending = false;
-    if (!h->stragglers.empty()) run_stragglers(h, cfg, in, out);
-    h->collectStragglers = false;
+    if (!run.stragglers.empty()) run_stragglers(h, run);
     return 0;
   } catch (const Err &e) {
     finish_tail(2);
-    h->collectStragglers = false;
     h->err = e.msg;
 #ifndef BATOTP_HOST_EMU
     cudaStreamSynchronize(h->copyStream);
@@ -2813,39 +2780,39 @@ int batotp_cuda_get_f64(batotp_handle h, const char *name, int traj, int row, do
 
 int batotp_cuda_set_max_steps(batotp_handle h, int n) {
   if (!h || n < 1024) return -1;
-  h->maxSteps = n;
+  h->opt.maxSteps = n;
   return 0;
 }
 
 int batotp_cuda_set_dyn_callback(batotp_handle h, batotp_dyn_fn fn, void *user) {
   if (!h) return -1;
-  h->dynFn = fn;
-  h->dynUser = user;
+  h->opt.dynFn = fn;
+  h->opt.dynUser = user;
   return 0;
 }
 
 int batotp_cuda_set_sweep_kernel(batotp_handle h, int mode) {
   if (!h || mode < 0 || mode > 2) return -1;
-  h->sweepKernel = mode;
+  h->opt.sweepKernel = mode;
   return 0;
 }
 
 int batotp_cuda_set_walker_kernel(batotp_handle h, int mode) {
   if (!h || mode < 0 || mode > 2) return -1;
-  h->walkerKernel = mode;
+  h->opt.walkerKernel = mode;
   return 0;
 }
 
 int batotp_cuda_set_step_hint(batotp_handle h, int n) {
   if (!h || n < 0) return -1;
-  h->stepHint = n;
+  h->opt.stepHint = n;
   h->hwSc = 0;  // the hint replaces what earlier chunks have learnt
   return 0;
 }
 
 int batotp_cuda_set_out_chunk(batotp_handle h, int n) {
   if (!h || n < 1) return -1;
-  h->outChunk = n;
+  h->opt.outChunk = n;
   return 0;
 }
 

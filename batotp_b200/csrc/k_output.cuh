@@ -123,6 +123,23 @@ __global__ void k_dyn_grid(WSP, Pmat pm, int npts, int nb) {
     for (int q = 0; q < w.AD; ++q) Ab[k * w.AD + q] = a[k][q];
 }
 
+// ----------------------------------------------------------------------------- output lengths
+// The output length of a trajectory follows from its forward sweep (tLast = tStep * (nFwd - 1)).  The plan kernels
+// below and the host's ragged layout (plan_ragged, which sizes each trajectory's block before the output phase runs)
+// both take it from here.
+// ba.cpp:1664-1706: oversampled length at the effective resolution and smoothing factor
+__host__ __device__ inline int out_n_over(double tLast, double outRes, double outSmooth) {
+  return imax_((int)(outSmooth * ceil(tLast / outRes + 1.)), 4);
+}
+// ba.cpp:1838-1871: length after smoothing and decimation (smoothing only when outSmooth > 1.5)
+__host__ __device__ inline int out_n_sm(int nOver, double outSmooth) {
+  return outSmooth > 1.5 ? imax_((int)((nOver - 1) / outSmooth) + 1, 4) : nOver;
+}
+// ba.cpp:1873-1921: final length (re-interpolated at the requested resolution outResT, or the smoothed rows as they are)
+__host__ __device__ inline int out_n_final(double tLast, double outResT, int isReinterp, int nSm) {
+  return isReinterp ? imax_((int)(ceil(tLast / outResT)), 4) : nSm;
+}
+
 // ----------------------------------------------------------------------------- output plan (T)
 // ba.cpp:1664-1706: output resolution bookkeeping, oversampled size, natural spline of sMVC(t), for every
 // trajectory of the resident chunk.  The output kernels after it work on the sub-chunk [w.b0, w.b0 + w.Bo).
@@ -140,8 +157,7 @@ __global__ void k_out_plan(WSP, ThomasTabs tabs) {
     outSmooth *= dmax_(outResT / outRes, 1.);
   }
   const double tLast = s.tStep * (double)(s.nFwd - 1);
-  int nOver = (int)(outSmooth * ceil(tLast / outRes + 1.));
-  nOver = imax_(nOver, 4);
+  const int nOver = out_n_over(tLast, outRes, outSmooth);
   s.isReinterp = isReinterp;
   s.outResEff = outRes;
   s.outSmooth = outSmooth;
@@ -444,14 +460,13 @@ __global__ void k_out_smooth_plan(WSP) {
   if (bl >= w.Bo) return;
   TrajState &s = w.st[w.b0 + bl];
   if (s.status & ST_FATAL_MASK) return;
+  s.nSm = out_n_sm(s.nOver, s.outSmooth);
   if (s.outSmooth > 1.5) {
     const int nIn = s.nOver;
-    s.nSm = imax_((int)((nIn - 1) / s.outSmooth) + 1, 4);
     int wv = imin_((int)s.outSmooth, nIn);
     const int wMid = wv / 2 + wv % 2 - 1;
     if (nIn < 2 * wMid + 1) s.status |= ST_UNSUPPORTED;  // degenerate window/length combination
-  } else
-    s.nSm = s.nOver;
+  }
 }
 
 // smooth + linear decimation of every row (src -> dst) and of the torque rows (TP over nSm).
@@ -675,12 +690,11 @@ __global__ void k_out_final_plan(WSP) {
   TrajState &s = w.st[w.b0 + bl];
   if (s.status & ST_FATAL_MASK) return;
   const double tLast = s.tStep * (double)(s.nFwd - 1);
+  s.nOut = out_n_final(tLast, s.outResT, s.isReinterp, s.nSm);
   if (s.isReinterp) {
-    s.nOut = imax_((int)(ceil(tLast / s.outResT)), 4);
     s.sresOut = s.outResT;
     s.nCartOut = CFG.c.robot_type == BATOTP_GENJNT ? s.nSm : s.nOut;
   } else {
-    s.nOut = s.nSm;
     s.sresOut = s.outResEff;
     s.nCartOut = s.nSm;
   }

@@ -51,6 +51,42 @@ class BatotpCfg(C.Structure):
         return c
 
 
+# The limit members of batotp_cfg in the order of struct batotp_limits (include/batotp_cuda.h): one row of 30 doubles
+LIMIT_FIELDS = (("jnt_vel_max", MAX_DOF), ("jnt_acc_max", MAX_DOF), ("jnt_trq_max", MAX_DOF), ("jnt_trq_min", MAX_DOF),
+                ("cart_vel_max", 1), ("cart_acc_max", 1))
+LIMIT_WIDTH = sum(n for _, n in LIMIT_FIELDS)
+
+
+def limit_row(cfg: BatotpCfg) -> np.ndarray:
+    """The limits of ``cfg`` as one float64 row of LIMIT_WIDTH values (batotp_limits order): scale it to build the
+    per-trajectory rows of a batch (``Context.make_in(..., limits=)``)."""
+    out = []
+    for nm, n in LIMIT_FIELDS:
+        v = getattr(cfg, nm)
+        out += list(v) if n > 1 else [v]
+    return np.array(out, dtype=np.float64)
+
+
+def with_limits(cfg: BatotpCfg, row) -> BatotpCfg:
+    """A copy of ``cfg`` whose limit members are replaced by ``row`` (LIMIT_WIDTH values, batotp_limits order), with
+    the config reader's rule for a NaN jnt_trq_min: what a trajectory of a batch with that row is computed under."""
+    row = np.asarray(row, dtype=np.float64).reshape(LIMIT_WIDTH)
+    c = cfg.copy()
+    k = 0
+    for nm, n in LIMIT_FIELDS:
+        if n > 1:
+            arr = getattr(c, nm)
+            for i in range(n):
+                arr[i] = float(row[k + i])
+        else:
+            setattr(c, nm, float(row[k]))
+        k += n
+    for i in range(MAX_DOF):
+        if math.isnan(c.jnt_trq_min[i]):
+            c.jnt_trq_min[i] = -c.jnt_trq_max[i]
+    return c
+
+
 def _payload_lines(path: str) -> List[str]:
     with open(path, "r") as f:
         return f.read().split("\n")

@@ -262,8 +262,10 @@ struct batotp_ctx {
     void *theta = nullptr, *cart = nullptr;
     double *ts = nullptr, *tres = nullptr;
     int *n0 = nullptr;
+    batotp_limits *lim = nullptr;  // [capInB] normalised limit rows (allocated once a batch carries them)
     size_t capTheta = 0, capCart = 0, capInB = 0, capInTs = 0;  // bytes (theta, cart), trajectories, timestamps
     std::vector<double> tresHost;
+    std::vector<batotp_limits> limHost;
     const batotp_batch_in *src = nullptr;  // what the set holds: chunk [first, first+B) of this batch
     int first = -1, B = 0;
     bool onCopyStream = false;
@@ -276,6 +278,7 @@ struct batotp_ctx {
   int curIn = 0;
   double *d_tres = nullptr;
   int *d_n0 = nullptr;
+  const batotp_limits *d_lim = nullptr;  // the bound set's limit rows, or NULL (w.lim from k_in_load on)
   bool copiesPending = false;  // row copies of the previous chunk may still be in flight on the copy stream
   const void *in_theta = nullptr, *in_cart = nullptr;  // device views used by k_in_load
   const double *in_ts = nullptr;
@@ -949,12 +952,19 @@ void launch_sweep_kernel(batotp_ctx *h, Kernel kern, int kind, int nt, size_t sm
   h->sweepLaunches++;
 }
 
+// (a chunk with limit rows runs the LIM instantiation, which reads each trajectory's own row)
 template <int J, bool CART, bool TRQ, bool PAR = false>
 void launch_sweep(batotp_ctx *h, bool group) {
-  if (group)
-    launch_sweep_kernel(h, k_sweep_group<J, CART, TRQ>, 2, SWG_NT, 0, GroupShape<J, CART>::G, "k_sweep_group");
+  constexpr size_t smem = SweepLayout<J, CART, TRQ, PAR>::bytes, smemLim = SweepLayout<J, CART, TRQ, PAR, true>::bytes;
+  constexpr int G = GroupShape<J, CART>::G;
+  if (group && h->w.lim)
+    launch_sweep_kernel(h, k_sweep_group<J, CART, TRQ, true>, 2, SWG_NT, 0, G, "k_sweep_group(limits)");
+  else if (group)
+    launch_sweep_kernel(h, k_sweep_group<J, CART, TRQ>, 2, SWG_NT, 0, G, "k_sweep_group");
+  else if (h->w.lim)
+    launch_sweep_kernel(h, k_sweep<J, CART, TRQ, PAR, true>, 1, SW_NT, smemLim, 1, "k_sweep(limits)");
   else
-    launch_sweep_kernel(h, k_sweep<J, CART, TRQ, PAR>, 1, SW_NT, SweepLayout<J, CART, TRQ, PAR>::bytes, 1, "k_sweep");
+    launch_sweep_kernel(h, k_sweep<J, CART, TRQ, PAR>, 1, SW_NT, smem, 1, "k_sweep");
 }
 
 // Which sweep kernel serves a chunk of B trajectories: one trajectory per lane (k_sweep.cuh: the fewest issue slots
@@ -973,7 +983,7 @@ int dispatch_sweep(batotp_ctx *h) {
   const DevCfg &c = h->cfg;
   const int key = c.J * 4 + (c.cartOn ? 2 : 0) + (c.trqOn ? 1 : 0);
   const bool par = c.trqOn && c.c.is_parallel && !c.c.is_par2ser;
-  const int capKey = key * 2 + (par ? 1 : 0);
+  const int capKey = (key * 2 + (par ? 1 : 0)) * 2 + (h->w.lim ? 1 : 0);
   if (capKey != h->sweepCapKey) {  // another kernel instance: its occupancy is not known yet
     h->sweepCap[0] = h->sweepCap[1] = 0;
     h->sweepCapKey = capKey;
@@ -1009,12 +1019,55 @@ int dispatch_sweep(batotp_ctx *h) {
 #include "host_strict.inl"
 namespace {
 // ---- phases ---------------------------------------------------------------------------
+// One trajectory's limit row as the kernels read it (batotp_cuda.h, batotp_limits): entries past nJoints take the cfg's
+// values, a NaN jnt_trq_min is -jnt_trq_max (ba.cpp:2020-2028), and a row with a used limit that is not finite, or a
+// velocity / acceleration maximum <= 0 of a limit that is on (or a velocity maximum the automatic step divides by),
+// is rejected: it is staged as NaN throughout, which k_in_load turns into
+// BATOTP_ST_UNSUPPORTED for its trajectory.  The float models of the filtered sweep kernel rely on positive, finite
+// maxima.  Returns false for a rejected row.
+bool normalise_limits(const batotp_cfg &c, const batotp_limits &in, batotp_limits &o) {
+  const int J = c.n_joints;
+  const bool auto_ = c.is_auto_integ_res != 0;
+  bool ok = true;
+  auto pos = [&](double v) { ok &= std::isfinite(v) && v > 0.0; };
+  auto nonneg = [&](double v) { ok &= std::isfinite(v) && v >= 0.0; };  // read by the automatic step only
+  for (int j = 0; j < MAXD; ++j) {
+    const bool used = j < J;
+    o.jnt_vel_max[j] = used ? in.jnt_vel_max[j] : c.jnt_vel_max[j];
+    o.jnt_acc_max[j] = used ? in.jnt_acc_max[j] : c.jnt_acc_max[j];
+    o.jnt_trq_max[j] = used ? in.jnt_trq_max[j] : c.jnt_trq_max[j];
+    o.jnt_trq_min[j] = used ? (std::isnan(in.jnt_trq_min[j]) ? -in.jnt_trq_max[j] : in.jnt_trq_min[j]) : c.jnt_trq_min[j];
+    if (!used) continue;
+    pos(o.jnt_vel_max[j]);
+    if (c.is_jnt_acc_on)
+      pos(o.jnt_acc_max[j]);
+    else if (auto_)
+      nonneg(o.jnt_acc_max[j]);
+    if (c.is_trq_on) ok &= std::isfinite(o.jnt_trq_max[j]) && std::isfinite(o.jnt_trq_min[j]);
+  }
+  o.cart_vel_max = in.cart_vel_max;
+  o.cart_acc_max = in.cart_acc_max;
+  if (c.is_cart_vel_on || auto_) pos(o.cart_vel_max);
+  if (c.is_cart_acc_on)
+    pos(o.cart_acc_max);
+  else if (auto_)
+    nonneg(o.cart_acc_max);
+  if (!ok) {
+    const double nan = std::nan("");
+    double *p = &o.jnt_vel_max[0];
+    for (size_t k = 0; k < sizeof(batotp_limits) / sizeof(double); ++k) p[k] = nan;
+  }
+  return ok;
+}
+
 void free_inset(batotp_ctx::InSet &q) {
   g_free(q.theta);
   g_free(q.cart);
   g_free(q.ts);
   g_free(q.tres);
   g_free(q.n0);
+  g_free(q.lim);
+  q.lim = nullptr;
   q.theta = q.cart = nullptr;
   q.ts = q.tres = nullptr;
   q.n0 = nullptr;
@@ -1042,7 +1095,8 @@ void issue_inputs(batotp_ctx *h, const batotp_batch_in *in, int first, int B, in
   // have been sized for another robot / path length: each block keeps its own capacity)
   const size_t needTh = (in->on_device || !th) ? 0 : thBytes, needCa = (in->on_device || !ca) ? 0 : caBytes;
   const size_t needTs = (in->on_device || !in->timestamp) ? 0 : (size_t)B * n0;
-  if (needTh > q.capTheta || needCa > q.capCart || (size_t)B > q.capInB || needTs > q.capInTs || !q.tres) {
+  if (needTh > q.capTheta || needCa > q.capCart || (size_t)B > q.capInB || needTs > q.capInTs || !q.tres ||
+      (in->limits && !q.lim)) {
     const size_t capB = std::max((size_t)B, q.capInB);
     const size_t cTh = std::max(needTh, q.capTheta), cCa = std::max(needCa, q.capCart), cTs = std::max(needTs, q.capInTs);
     free_inset(q);
@@ -1051,6 +1105,7 @@ void issue_inputs(batotp_ctx *h, const batotp_batch_in *in, int first, int B, in
     if (cTs) q.ts = (double *)g_alloc(cTs * 8);
     q.tres = (double *)g_alloc(capB * 8);
     q.n0 = (int *)g_alloc(capB * 4);
+    if (in->limits) q.lim = (batotp_limits *)g_alloc(capB * sizeof(batotp_limits));
     q.capTheta = cTh;
     q.capCart = cCa;
     q.capInB = capB;
@@ -1059,6 +1114,11 @@ void issue_inputs(batotp_ctx *h, const batotp_batch_in *in, int first, int B, in
   q.tresHost.resize(B);
   for (int b = 0; b < B; ++b) q.tresHost[b] = in->tres ? in->tres[first + b] : in->tres_all;  // per-trajectory tres (small)
   g_h2d(q.tres, q.tresHost.data(), (size_t)B * 8, st);
+  if (in->limits) {
+    q.limHost.resize(B);
+    for (int b = 0; b < B; ++b) normalise_limits(c.c, in->limits[first + b], q.limHost[b]);
+    g_h2d(q.lim, q.limHost.data(), (size_t)B * sizeof(batotp_limits), st);
+  }
   if (!in->on_device) {
     if (th) g_h2d(q.theta, (const char *)th + (size_t)first * c.J * n0 * es, thBytes, st);
     if (ca) g_h2d(q.cart, (const char *)ca + (size_t)first * c.Cin * n0 * es, caBytes, st);
@@ -1106,6 +1166,7 @@ void stage_inputs(batotp_ctx *h, const batotp_batch_in *in, int first, int B) {
   }
   h->d_tres = q.tres;
   h->d_n0 = q.n0;
+  h->d_lim = in->limits ? q.lim : nullptr;
   h->B = B;
   h->n0max = n0;
 }
@@ -1113,6 +1174,7 @@ void stage_inputs(batotp_ctx *h, const batotp_batch_in *in, int first, int B) {
 void run_load_prepare(batotp_ctx *h, bool haveN0) {
   Ws &w = h->w;
   w.B = h->B;
+  w.lim = h->d_lim;
   const int *n0 = haveN0 ? h->d_n0 : nullptr;
   if (h->inF64)
     LAUNCH_TP(h, (k_in_load<double>), h->n0max, h->B, w, (const double *)h->in_theta, (const double *)h->in_cart, n0,
@@ -2410,6 +2472,7 @@ static void run_stragglers(batotp_handle h, BatchRun &r) {
   std::vector<char> hTh, hCa;
   std::vector<double> hTs, hTres(n);
   std::vector<int> hN0(n);
+  std::vector<batotp_limits> hLim(in->limits ? n : 0);
   void *dTh = nullptr, *dCa = nullptr;
   double *dTs = nullptr;
   struct Guard {
@@ -2434,6 +2497,7 @@ static void run_stragglers(batotp_handle h, BatchRun &r) {
     const size_t g = (size_t)idx[k];
     hTres[k] = in->tres ? in->tres[g] : in->tres_all;
     hN0[k] = in->n0 ? in->n0[g] : n0;
+    if (in->limits) hLim[k] = in->limits[g];
     if (in->on_device) {
       if (th) g_d2d((char *)dTh + k * thRow, (const char *)th + g * thRow, thRow, h->stream);
       if (ca) g_d2d((char *)dCa + k * caRow, (const char *)ca + g * caRow, caRow, h->stream);
@@ -2448,6 +2512,7 @@ static void run_stragglers(batotp_handle h, BatchRun &r) {
   in2.B = n;
   in2.n0 = in->n0 ? hN0.data() : nullptr;
   in2.tres = hTres.data();
+  in2.limits = in->limits ? hLim.data() : nullptr;
   const void *pTh = in->on_device ? dTh : (th ? (void *)hTh.data() : nullptr);
   const void *pCa = in->on_device ? dCa : (ca ? (void *)hCa.data() : nullptr);
   in2.theta_f32 = f64 ? nullptr : (const float *)pTh;

@@ -197,7 +197,8 @@ __global__ void k_in_load(WSP, const T *theta, const T *cart, const int *n0, con
   const int n = n0 ? n0[b] : n0max;
   if (i == 0) {
     TrajState &s = w.st[b];
-    s.status = 0;
+    // a limit row the host rejected (NaN throughout) keeps its trajectory out of every stage
+    s.status = (w.lim && w.lim[b].jnt_vel_max[0] != w.lim[b].jnt_vel_max[0]) ? ST_UNSUPPORTED : 0;
     s.nPts = n;
     s.tresInput = tres[b];
     s.sres = tres[b];
@@ -250,6 +251,7 @@ __global__ void k_in_prepare(WSP, const double *ts, int n0max, int hasTheta, int
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= w.B) return;
   TrajState &s = w.st[b];
+  if (s.status & ST_FATAL_MASK) return;  // (a rejected limit row, k_in_load)
   const int J = CFG.J, R = CFG.R;
   int nPts = s.nPts;
   const RV scr = RV{w.nrm + (size_t)b * 2, (size_t)w.B * 2};  // per-trajectory scratch vector
@@ -574,6 +576,14 @@ __global__ void k_adjust_inc(WSP, int npts, int nb) {
   o[1] = sqrt(dcartSQ);
 }
 
+// the limit part of the automatic integration step (ba.cpp:493-556); lim: batotp_cfg or batotp_limits
+template <class LT>
+__host__ __device__ __forceinline__ double auto_integ_res(const LT &lim, int J, double K) {
+  double r = K * lim.cart_acc_max / lim.cart_vel_max;
+  for (int i = 0; i < J; ++i) r = dmax_(r, K * lim.jnt_acc_max[i] / lim.jnt_vel_max[i]);
+  return r;
+}
+
 __global__ void k_adjust_s(WSP, int special, int haveInc) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= w.B) return;
@@ -673,8 +683,8 @@ __global__ void k_adjust_s(WSP, int special, int haveInc) {
     double thetaRat = tnLast;
     if (!CFG.c.are_jnt_deg) thetaRat *= RAD2DEG;
     const double minIntegRes = 0.004, maxIntegRes = 0.2, K = 0.0003;
-    double newIntegRes = K * CFG.c.cart_acc_max / CFG.c.cart_vel_max;
-    for (int i = 0; i < J; ++i) newIntegRes = dmax_(newIntegRes, K * CFG.c.jnt_acc_max[i] / CFG.c.jnt_vel_max[i]);
+    // from the trajectory's own limit row when the batch has them
+    double newIntegRes = w.lim ? auto_integ_res(w.lim[b], J, K) : auto_integ_res(CFG.c, J, K);
     newIntegRes = dmin_(newIntegRes, maxIntegRes);
     const double changeRat = cartRat / thetaRat;
     double jointIntegRes = maxIntegRes * changeRat * changeRat;

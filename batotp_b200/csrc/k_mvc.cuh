@@ -7,7 +7,8 @@
 #pragma once
 #include "k_sweep.cuh"
 
-template <int J, bool CART, bool TRQ>
+// LIM: trajectory b's limit row (w.lim) instead of the cfg's limits
+template <int J, bool CART, bool TRQ, bool LIM = false>
 __global__ void k_mvc(WSP, double sdotStart, double *out, int cap, int npts, int nb) {
   TP_DECOMP(nb);
   if (i >= npts) return;
@@ -19,8 +20,9 @@ __global__ void k_mvc(WSP, double sdotStart, double *out, int cap, int npts, int
   constexpr int RT = NK + (TRQ ? 4 * J : 0);
   const double absh = s.integRes;
   const double sBack = s.sresC * (double)(s.nPtsC - 1);
+  const auto &lim = LimSrc<LIM>::get(w, LIM ? w.lim + b : nullptr);
   TrajConsts C;
-  traj_consts(C, CFG, s, sBack, absh);
+  traj_consts(C, CFG, lim, s, sBack, absh);
   int seg = imin_(i, s.nPtsC - 2);
   const double sCur = s.sresC * (double)i;
   double sSeg;
@@ -36,7 +38,7 @@ __global__ void k_mvc(WSP, double sdotStart, double *out, int cap, int npts, int
   };
   const KGlobal K{w.tab + ((size_t)b * w.Nc + seg) * (size_t)RT * 4};
   PointVals<J, CART, TRQ> P;
-  eval_point<J, CART, TRQ>(P, K, tau, C, CFG);
+  eval_point<J, CART, TRQ>(P, K, tau, C, CFG, lim);
   // sdotLim without the MVC term and with _sdotMin = 0
   double sd = sdotStart;
   sd = dmin_(sd, sBack / absh);
@@ -46,7 +48,7 @@ __global__ void k_mvc(WSP, double sdotStart, double *out, int cap, int npts, int
   bis.begin(sd);
   double Lo, Hi;
   for (;;) {
-    const bool viol = verify_point<J, CART, TRQ>(P, C, CFG, bis.sdotCur, Lo, Hi);
+    const bool viol = verify_point<J, CART, TRQ>(P, C, CFG, lim, bis.sdotCur, Lo, Hi);
     if (bis.step(viol) != 0) break;
   }
   out[(size_t)b * cap + i] = bis.sdotIn;

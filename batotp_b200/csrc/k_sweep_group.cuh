@@ -61,7 +61,9 @@ __device__ __forceinline__ double group_max(double v, int lane) {
   return v;
 }
 
-template <int J, bool CART, bool TRQ>
+// LIM: every trajectory has its own limit row (w.lim): a lane loads its joint's four values and the Cartesian ones when
+// its group picks a trajectory up
+template <int J, bool CART, bool TRQ, bool LIM = false>
 __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
   constexpr int G = GroupShape<J, CART>::G;
   constexpr int NK = J + (CART ? 3 : 0);
@@ -83,8 +85,11 @@ __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
 #define SDD(k) sS[7 + (k)][tid]
   // this lane's limits
   const int jj = jointLane ? gl : 0;
-  const double velMax = CFG.c.jnt_vel_max[jj], accMax = CFG.c.jnt_acc_max[jj];
-  const double trqMax = CFG.c.jnt_trq_max[jj], trqMin = CFG.c.jnt_trq_min[jj];
+  const batotp_limits *lrow = nullptr;  // LIM: the row of trajectory b
+#define LIMS LimSrc<LIM>::get(w, lrow)
+  double velMax = CFG.c.jnt_vel_max[jj], accMax = CFG.c.jnt_acc_max[jj];
+  double trqMax = CFG.c.jnt_trq_max[jj], trqMin = CFG.c.jnt_trq_min[jj];
+  double cartVelMax = CFG.c.cart_vel_max;
   const bool accOn = CFG.c.is_jnt_acc_on != 0, cartAccOn = CART && CFG.c.is_cart_acc_on != 0;
   const bool cartVelOn = CART && CFG.c.is_cart_vel_on != 0;
 
@@ -136,7 +141,7 @@ __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
     lastSeg = s.nPtsC - 2;
     sBack = s.sresC * (double)(s.nPtsC - 1);
     sdotCap = sBack / absh;
-    traj_consts(C, CFG, s, sBack, absh);
+    traj_consts(C, CFG, LIMS, s, sBack, absh);
     tab = w.tab + (size_t)b * w.Nc * (size_t)w.RT * 4;
     double *hb = w.hist + (size_t)b * 4 * w.Sc;
     if (d == 1) {
@@ -190,6 +195,16 @@ __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
           status = 0;
           nVerify = 0;
           sLastSec = w.st[b].sLastSec;
+          if (LIM) {
+            lrow = w.lim + b;
+            velMax = lrow->jnt_vel_max[jj];
+            accMax = lrow->jnt_acc_max[jj];
+            if (TRQ) {
+              trqMax = lrow->jnt_trq_max[jj];
+              trqMin = lrow->jnt_trq_min[jj];
+            }
+            if (CART) cartVelMax = lrow->cart_vel_max;
+          }
           sweep_begin(-1, 0);
         }
       }
@@ -444,7 +459,7 @@ __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
         Q1 = 2 * (vx * ax + vy * ay + vz * az);
         Q2 = ax * ax + ay * ay + az * az;
         r2A = sdiv::prep(2 * Q0);
-        if (cartVelOn && Q0 > C.thrQ) vl = dmin_(vl, CFG.c.cart_vel_max / sqrt(Q0));
+        if (cartVelOn && Q0 > C.thrQ) vl = dmin_(vl, cartVelMax / sqrt(Q0));
       }
       if (TRQ) {  // ba.cpp:1387-1405
         const double tau3 = tau2 * tau;
@@ -571,4 +586,5 @@ __global__ void __launch_bounds__(SWG_NT) k_sweep_group(WSP) {
   }
 #undef SD
 #undef SDD
+#undef LIMS
 }

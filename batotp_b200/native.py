@@ -12,7 +12,7 @@ from typing import Optional
 
 import numpy as np
 
-from .config import BatotpCfg
+from .config import LIMIT_WIDTH, BatotpCfg
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libbatotp_cuda.so")
@@ -26,10 +26,22 @@ ST_FATAL_MASK = 1 | 2 | 4 | 8 | 16 | 32 | 64 | 256 | 512
 ST_BISECT_FAIL = 128
 
 
+class Limits(C.Structure):
+    """struct batotp_limits: one trajectory's limits (the limit members of batotp_cfg)."""
+    _fields_ = [("jnt_vel_max", C.c_double * 7), ("jnt_acc_max", C.c_double * 7), ("jnt_trq_max", C.c_double * 7),
+                ("jnt_trq_min", C.c_double * 7), ("cart_vel_max", C.c_double), ("cart_acc_max", C.c_double)]
+
+
+# numpy image of struct batotp_limits (a [B] array of it is a valid `limits` argument)
+LIMITS_DTYPE = np.dtype([(nm, np.float64, (7,)) if nm.startswith("jnt") else (nm, np.float64)
+                         for nm, _ in Limits._fields_])
+
+
 class BatchIn(C.Structure):
     _fields_ = [("B", C.c_int), ("n0_max", C.c_int), ("n0", _ip), ("tres", _dp), ("tres_all", C.c_double),
                 ("theta_f32", C.c_void_p), ("cart_f32", C.c_void_p), ("theta_f64", C.c_void_p),
-                ("cart_f64", C.c_void_p), ("timestamp", C.c_void_p), ("on_device", C.c_int)]
+                ("cart_f64", C.c_void_p), ("timestamp", C.c_void_p), ("on_device", C.c_int),
+                ("limits", C.POINTER(Limits))]
 
 
 class BatchOut(C.Structure):
@@ -337,9 +349,11 @@ class Context:
         return ms.value
 
     @staticmethod
-    def make_in(theta=None, cart=None, tres=0.01, n0=None, timestamp=None, device_ptrs=None) -> BatchIn:
+    def make_in(theta=None, cart=None, tres=0.01, n0=None, timestamp=None, device_ptrs=None, limits=None) -> BatchIn:
         """theta/cart: numpy [B, rows, n0_max] float32 or float64 (C-contiguous).
-        device_ptrs: optional dict(theta=int, cart=int, B=, n0_max=, f64=bool) for HBM-resident inputs."""
+        device_ptrs: optional dict(theta=int, cart=int, B=, n0_max=, f64=bool) for HBM-resident inputs.
+        limits: optional per-trajectory limits, a [B] array of LIMITS_DTYPE or a [B, 30] float64 array in
+        batotp_limits order (config.limit_row); always host memory."""
         bi = BatchIn()
         keep = []
         if device_ptrs:
@@ -376,6 +390,18 @@ class Context:
             ts = np.ascontiguousarray(timestamp, dtype=np.float64)
             keep.append(ts)
             bi.timestamp = ts.ctypes.data
+        if limits is not None:
+            lim = np.asarray(limits)
+            if lim.dtype == LIMITS_DTYPE:
+                lim = np.ascontiguousarray(lim)
+            else:
+                lim = np.ascontiguousarray(lim, dtype=np.float64)
+                if lim.ndim != 2 or lim.shape[1] != LIMIT_WIDTH:
+                    raise ValueError("limits: a [B] array of LIMITS_DTYPE or a [B, %d] float64 array" % LIMIT_WIDTH)
+            if lim.shape[0] != bi.B:
+                raise ValueError("limits: %d rows for %d trajectories" % (lim.shape[0], bi.B))
+            keep.append(lim)
+            bi.limits = lim.ctypes.data_as(C.POINTER(Limits))
         bi._keep = keep
         return bi
 

@@ -119,6 +119,28 @@ typedef void (*batotp_dyn_fn)(void *user, int n_joints, const double *theta, con
                               const double *thetaD2, double *a1, double *a2, double *a3, double *a4);
 int batotp_cuda_set_dyn_callback(batotp_handle h, batotp_dyn_fn fn, void *user);
 
+/* ---- per-trajectory limits ------------------------------------------------------------------
+ * The limit members of batotp_cfg, for one trajectory (same names, same meaning).  A batch that carries one row per
+ * trajectory gives trajectory b exactly the results of a run whose configuration is the batch cfg with these members
+ * replaced by row b.  Everything else stays batch-wide: the on/off flags (is_jnt_acc_on, is_cart_*_on, is_trq_on),
+ * resolutions, thresholds, integ_res, max_integ_time, the robot and the dynamic model.  Rules, per row:
+ *  - entries at j >= n_joints are ignored;
+ *  - a NaN jnt_trq_min[j] means -jnt_trq_max[j] (the config reader's rule, ba.cpp:2020-2028);
+ *  - the limits the configuration uses must be finite and, for velocity and acceleration maxima, > 0: jnt_vel_max
+ *    always (sdotLim applies it, ba.cpp:1219); jnt_acc_max with is_jnt_acc_on; jnt_trq_max / min with is_trq_on;
+ *    cart_vel_max / cart_acc_max with is_cart_vel_on / is_cart_acc_on.  With is_auto_integ_res the automatic step
+ *    is formed from acc / vel quotients of all of them (ba.cpp:493-556): cart_vel_max must then be > 0 and the
+ *    acceleration maxima of limits that are off finite and >= 0.  A row that breaks this marks its trajectory
+ *    BATOTP_ST_UNSUPPORTED (no output); the rest of the batch goes on. */
+typedef struct batotp_limits {
+  double jnt_vel_max[BATOTP_MAX_DOF];
+  double jnt_acc_max[BATOTP_MAX_DOF];
+  double jnt_trq_max[BATOTP_MAX_DOF];
+  double jnt_trq_min[BATOTP_MAX_DOF];
+  double cart_vel_max;
+  double cart_acc_max;
+} batotp_limits;
+
 /* ---- batch input: what BA::loadTrajectoryData leaves in Traj (ba.cpp:2206-2461) -------- */
 typedef struct batotp_batch_in {
   int B;                  /* trajectories */
@@ -134,6 +156,7 @@ typedef struct batotp_batch_in {
   const double *cart_f64;
   const double *timestamp; /* [B][n0_max] CSV timestamps or NULL (ba.cpp:98-127) */
   int on_device;           /* 1: the payload pointers are device pointers already resident in HBM */
+  const batotp_limits *limits; /* [B] limits per path, or NULL: the cfg's for all   (always a HOST pointer) */
 } batotp_batch_in;
 
 /* ---- batch output: what BA::writeOutputData would serialise (ba.cpp:2510-2759) --------- */
@@ -181,6 +204,7 @@ int batotp_cuda_optimize_batch(batotp_handle h, const batotp_cfg *cfg, const bat
  * _interp_input = BA::interpInputData (ba.cpp:95), _sweeps = BA::sweep x2 (ba.cpp:979; the
  * reverse pass must precede the forward pass, so both run in one launch),
  * _interp_output = BA::interpOutputData (ba.cpp:1661), _fetch = copy results out. */
+/* (batotp_cuda_load honours in->limits: the later phases and batotp_cuda_mvc_per_sample use the rows) */
 int batotp_cuda_load(batotp_handle h, const batotp_cfg *cfg, const batotp_batch_in *in);
 int batotp_cuda_interp_input(batotp_handle h);
 int batotp_cuda_sweeps(batotp_handle h);
